@@ -12,7 +12,10 @@ One bench *step* = one reverse-diffusion step of the whole batch: score call, th
     value [samples/s] = n_gpus * batch / (100 * seconds_per_step).
 Multi-GPU: one process per GPU, the sample batch is sharded, no data-path collective (weak scaling).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the predictor returned in the last timed step (x_next, xhat0) as float32 .npy files;
+the inputs depend only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import functools
@@ -58,7 +61,32 @@ def parse():
                     help='skip the config 3 / 4 / 5 blocks (stack_501, hot_path_sweep, adapted)')
     ap.add_argument('--cpu-threads', type=int, default=0,
                     help='host threads of the CPU reference arm (0 = every core this process may use)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='write the outputs of the last timed step (x_next, xhat0) to DIR/<name>.npy, for either '
+                         '--impl (float32, at most 64 MB in all)')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    return args
+
+
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(out_dir, arrays, rank=0, world=1):
+    """Save the [batch, ...] tensors of `arrays` as float32 DIR/<name>.npy (suffix _rank<r> when sharded).  When they
+    would exceed DUMP_BYTES over all ranks, the same seeded subset of samples is kept in every array."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = next(iter(arrays.values())).shape[0]
+    per_sample = sum(4 * t[0].numel() for t in arrays.values())
+    keep = min(n, DUMP_BYTES // world // per_sample)
+    assert keep > 0, 'one sample of the outputs (%d bytes) exceeds the dump limit of %d bytes per rank' \
+        % (per_sample, DUMP_BYTES // world)
+    idx = None if keep == n else torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, keep, replace=False)))
+    suffix = '_rank%d' % rank if world > 1 else ''
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        np.save(os.path.join(out_dir, name + suffix + '.npy'), (t if idx is None else t[idx]).numpy())
 
 
 def peaks():
@@ -175,7 +203,8 @@ def cpu_reference_arm(args, steps, warmup, quiet=False):
     """The reference's CPU path for one reverse step at batch 1 (its MatmulRayTrafo handles one
     image per call, reference src/physics/matmul_ray_trafo.py:108-109): torch.sparse.mm projector
     + the reference's cg / Tweedie / ddim recurrences + the same UNet on the host cores.
-    Uses the reference's own code when the checkout is present, else the oracle port."""
+    Uses the reference's own code when SCD_REFERENCE_ROOT names a checkout of it, else the oracle port.  Returns the
+    timings and, under 'outputs', what the last timed step returned (x_next, xhat0)."""
     from oracle import oracle as O
     from oracle import ref_harness
     from bench_support.phantoms import disk_ellipses
@@ -204,18 +233,18 @@ def cpu_reference_arm(args, steps, warmup, quiet=False):
 
         def one(x, t, tp):
             return ref_dds(score=score, sde=sde, x=x, rhs=atb, time_step=(torch.ones(1) * t, torch.ones(1) * tp),
-                           eta=ETA, gamma=GAMMA, step_size=1, cg_kwargs={'max_iter': CG_ITER}, ray_trafo=ort)[0]
+                           eta=ETA, gamma=GAMMA, step_size=1, cg_kwargs={'max_iter': CG_ITER}, ray_trafo=ort)
     else:
         abar = O.ref_port_alpha_bar()
 
         def one(x, t, tp):
             return O.ref_port_dds_step(score, x, atb, abar, torch.ones(1) * t, torch.ones(1) * tp, GAMMA, ETA,
-                                       CG_ITER, ort)[0]
+                                       CG_ITER, ort)
     for i in range(warmup):
-        x = one(x, *pairs[i % len(pairs)])
+        x, xm = one(x, *pairs[i % len(pairs)])
     t0 = time.perf_counter()
     for i in range(steps):
-        x = one(x, *pairs[(warmup + i) % len(pairs)])
+        x, xm = one(x, *pairs[(warmup + i) % len(pairs)])
     dt = (time.perf_counter() - t0) / max(steps, 1)
     # projector alone, for the per-operator comparison
     ta = time.perf_counter(); ort(x); ta = time.perf_counter() - ta
@@ -231,16 +260,17 @@ def cpu_reference_arm(args, steps, warmup, quiet=False):
                       'CG/DDIM on host; %.2f s/step; A %.3f s, A* %.3f s per apply'
                       % (steps, REVERSE_STEPS, args.unet, dt, ta, tb),
             'seconds_per_step': dt, 'fp_seconds': ta, 'bp_seconds': tb,
-            'dc_seconds': dc}
+            'dc_seconds': dc, 'outputs': {'x_next': x, 'xhat0': xm}}
 
 
 def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 5))          # bounded: each CPU step takes seconds
-    warm = max(0, min(args.warmup, 1))
+    steps, warm = args.steps, args.warmup
     cb = cpu_reference_arm(args, steps, warm)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cb['outputs'])
     line = {
         'impl': 'reference', 'metric': 'SCD samples/sec at 256^2', 'value': cb['value'], 'unit': 'samples/s',
         'n_gpus': args.gpus, 'steps': steps, 'warmup': warm, 'ms_per_step': cb['seconds_per_step'] * 1e3,
@@ -393,6 +423,8 @@ def run_b200(args):
         e1.record()
         barrier()
     launches = fused.launch_count()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'x_next': x, 'xhat0': xm}, rank, world)
     ms_total = e0.elapsed_time(e1)
     tt = torch.tensor([ms_total], device=dev)
     if world > 1:

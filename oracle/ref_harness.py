@@ -2,8 +2,9 @@
 third-party dependencies stubbed, so that its cg / ddim / apTweedy / DDPM /
 predictors / BaseSampler / MatmulRayTrafo run verbatim on CPU.
 
-TEST INFRASTRUCTURE ONLY, and only usable where the reference checkout exists
-(the authoring container).  Used by tests/golden/make_golden.py to generate the
+TEST INFRASTRUCTURE ONLY, and only usable where the environment variable
+SCD_REFERENCE_ROOT names a checkout of the reference project (it is not part of
+this repository).  Used by tests/golden/make_golden.py to generate the
 committed golden vectors and by tests marked `needs_reference`.
 Recipe: SURVEY.md Appendix B.
 """
@@ -11,11 +12,11 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get('SCD_REFERENCE_ROOT', '/root/reference')
+REFERENCE_ROOT = os.environ.get('SCD_REFERENCE_ROOT', '')
 
 
 def available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, 'src'))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, 'src'))
 
 
 def _stub(name, **attrs):
@@ -28,7 +29,8 @@ def _stub(name, **attrs):
 def import_reference():
     """Returns the reference's ``src`` package."""
     if not available():
-        raise RuntimeError('reference checkout not found at %s' % REFERENCE_ROOT)
+        raise RuntimeError('no reference checkout: set SCD_REFERENCE_ROOT to the directory that holds its src/ '
+                           '(now %r)' % REFERENCE_ROOT)
     if 'src' in sys.modules and getattr(sys.modules['src'], '__scd_ref__', False):
         return sys.modules['src']
 

@@ -14,7 +14,7 @@ GOLDEN = os.path.join(ROOT, 'tests', 'golden')
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (B200); run with -m gpu')
-    config.addinivalue_line('markers', 'needs_reference: needs the reference checkout at /root/reference')
+    config.addinivalue_line('markers', 'needs_reference: needs the reference checkout named by SCD_REFERENCE_ROOT')
 
 
 def pytest_collection_modifyitems(config, items):
@@ -25,7 +25,7 @@ def pytest_collection_modifyitems(config, items):
         if 'gpu' in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason='no CUDA device'))
         if 'needs_reference' in item.keywords and not ref_harness.available():
-            item.add_marker(pytest.mark.skip(reason='reference checkout not present'))
+            item.add_marker(pytest.mark.skip(reason='SCD_REFERENCE_ROOT names no reference checkout'))
 
 
 @pytest.fixture(scope='session')

@@ -1,7 +1,7 @@
 """Generate the golden vectors under tests/golden/ by running the REFERENCE's own code.
 
-Run in the authoring container (needs /root/reference):
-    python tests/golden/make_golden.py
+Needs a checkout of the reference project, named by SCD_REFERENCE_ROOT:
+    SCD_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py
 
 The reference package is imported through oracle/ref_harness.py (third-party imports
 stubbed).  Its cg, apTweedy, ddim, DDPM, _schedule_jump, DDS predictor and BaseSampler

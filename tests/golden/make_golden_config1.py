@@ -10,7 +10,7 @@ src.samplers.utils.decomposed_diffusion_sampling_sde_predictor (which calls the 
 on CPU.  The projector it calls is the C oracle (oracle/ray_oracle.c) behind a small torch adapter, because the
 reference's own projector (ODL/ASTRA) cannot run here.
 
-    python tests/golden/make_golden_config1.py        # ~10 min on 8 cores; writes tests/golden/config1_256.npz
+    SCD_REFERENCE_ROOT=<checkout> python tests/golden/make_golden_config1.py    # ~10 min on 8 cores; writes tests/golden/config1_256.npz
 
 Stored per image i: gt_i (fp32), y_i (noisy sinogram made by the reference's `simulate`), fbp-free;
 psnr_i of the reference reconstruction; recon_i in full for i < 3 and as 4x4 block means for all i.

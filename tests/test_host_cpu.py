@@ -428,23 +428,6 @@ def test_simulate_reproduces_the_reference_measurements(golden):
     assert abs(level - 0.01 * float(ort(gt).abs().mean())) < 1e-12
 
 
-@pytest.mark.needs_reference
-def test_simulate_and_dataset_equal_the_reference_code():
-    from oracle import ref_harness
-    ref_harness.import_reference()
-    from src.physics.simulation import simulate as ref_simulate, SimulatedDataset as RefDataset
-    rt = _MatrixTrafo()
-    g = torch.Generator().manual_seed(4)
-    x = torch.rand(3, 1, 6, 5, generator=g)
-    a = ref_simulate(x, rt, 0.05, rng=np.random.default_rng(7))
-    b = pkg.simulate(x, rt, 0.05, rng=np.random.default_rng(7))
-    assert torch.equal(a, b)
-    imgs = [torch.rand(1, 6, 5, generator=g) for _ in range(3)]
-    for k, (ra, rb) in enumerate(zip(RefDataset(imgs, rt, 0.05), pkg.SimulatedDataset(imgs, rt, 0.05))):
-        for u, v in zip(ra, rb):
-            assert torch.equal(u, v), k
-
-
 def test_simulated_dataset_and_get_data_from_ground_truth():
     rt = _MatrixTrafo()
     g = torch.Generator().manual_seed(5)
@@ -543,3 +526,58 @@ def test_bench_build_id_and_reference_arm_helpers():
     assert bench.host_cores() >= 1
     pairs = bench.time_pairs()
     assert len(pairs) == 100 and pairs[0] == (990, 980) and pairs[-1] == (0, -1)
+
+
+def test_bench_dump_outputs_float32_within_the_size_cap(tmp_path, monkeypatch):
+    """--dump-outputs: one float32 .npy per returned array; above the cap the same seeded subset of samples is kept in
+    every array, and the subset does not change from run to run."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location('bench_mod', os.path.join(ROOT, 'bench.py'))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    a = torch.arange(6 * 2 * 3, dtype=torch.float64).reshape(6, 1, 2, 3)
+    bench.dump_outputs(str(tmp_path / 'full'), {'x_next': a, 'xhat0': -a})
+    x, h = np.load(tmp_path / 'full' / 'x_next.npy'), np.load(tmp_path / 'full' / 'xhat0.npy')
+    assert x.dtype == np.float32 and np.array_equal(x, a.numpy()) and np.array_equal(h, -a.numpy())
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 3 * 2 * 4 * 6)            # room for 3 of the 6 samples of both arrays
+    for d in ('s1', 's2'):
+        bench.dump_outputs(str(tmp_path / d), {'x_next': a, 'xhat0': -a}, rank=1, world=1)
+    xs, hs = np.load(tmp_path / 's1' / 'x_next.npy'), np.load(tmp_path / 's1' / 'xhat0.npy')
+    assert xs.shape == (3, 1, 2, 3) and np.array_equal(hs, -xs)
+    assert np.array_equal(xs, np.load(tmp_path / 's2' / 'x_next.npy'))
+    assert all(any(np.array_equal(r, s) for s in a.numpy()) for r in xs)
+    bench.dump_outputs(str(tmp_path / 'r'), {'x_next': a}, rank=1, world=2)
+    assert sorted(os.listdir(tmp_path / 'r')) == ['x_next_rank1.npy']
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 4 * 6 - 1)                 # not even one sample fits: refused
+    with pytest.raises(AssertionError, match='dump limit'):
+        bench.dump_outputs(str(tmp_path / 'e'), {'x_next': a})
+
+
+def test_bench_reference_arm_honours_steps_and_dumps(tmp_path, monkeypatch, capsys):
+    """--steps sets the number of timed steps of the CPU reference arm too (it is not clamped), --steps < 1 is
+    refused, and --dump-outputs writes the arm's last (x_next, xhat0)."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location('bench_mod', os.path.join(ROOT, 'bench.py'))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    for bad in (['--steps', '0'], ['--warmup', '-1']):
+        monkeypatch.setattr('sys.argv', ['bench.py'] + bad)
+        with pytest.raises(SystemExit):
+            bench.parse()
+    calls = []
+    arm = bench.cpu_reference_arm
+    monkeypatch.setattr(bench, 'cpu_reference_arm', lambda a, s, w: calls.append((s, w)) or arm(a, s, w))
+    monkeypatch.setattr('sys.argv', ['bench.py', '--impl', 'reference', '--unet', 'small', '--steps', '1', '--warmup',
+                                     '2', '--dump-outputs', str(tmp_path)])
+    capsys.readouterr()
+    grad, threads = torch.is_grad_enabled(), torch.get_num_threads()
+    try:
+        bench.run_reference(bench.parse())
+    finally:                                    # the arm switches autograd off and sets the thread count process-wide
+        torch.set_grad_enabled(grad)
+        torch.set_num_threads(threads)
+    line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
+    assert calls == [(1, 2)] and line['steps'] == 1 and line['warmup'] == 2
+    for n in ('x_next', 'xhat0'):
+        v = np.load(tmp_path / (n + '.npy'))
+        assert v.shape == (1, 1, 256, 256) and v.dtype == np.float32 and np.isfinite(v).all()
