@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from conftest import rel_l2
+from fp64_reference import cg64
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -53,28 +54,6 @@ def test_tweedie_rhs_fused_b(golden):
     assert torch.equal(b, xh + 0.01 * atb)
 
 
-def _cg_fp64(geom, x0, rhs, gamma, k):
-    """The same CG recurrences in float64 on the oracle matrices: the exact-arithmetic arbiter."""
-    J = O.joseph_matrix(geom)
-    Bm = O.bp_matrix(geom)
-    nb = x0.shape[0]
-    X = x0.reshape(nb, -1).T.astype(np.float64)
-    R = rhs.reshape(nb, -1).T.astype(np.float64)
-    op = lambda v: v + gamma * (Bm @ (J @ v))       # noqa: E731
-    r = R - op(X)
-    p = r.copy()
-    rr = (r * r).sum(0)
-    for _ in range(k):
-        d = op(p)
-        alpha = rr / (p * d).sum(0)
-        X = X + alpha * p
-        r = r - alpha * d
-        rr_new = (r * r).sum(0)
-        p = r + (rr_new / rr) * p
-        rr = rr_new
-    return X.T.reshape(x0.shape)
-
-
 @pytest.mark.parametrize('gamma', [0.01, 1.0])
 def test_cg_matches_reference_cg(golden, gamma):
     """Fused scd_cg vs the reference's cg() run on the oracle operator (golden), every n_iter.
@@ -93,7 +72,7 @@ def test_cg_matches_reference_cg(golden, gamma):
         ref = d['x_g%g_k%d' % (gamma, k)]
         err = rel_l2(x, ref)
         if err >= 1e-5:
-            exact = _cg_fp64(geom, d['x0'], d['rhs'], gamma, k)
+            exact = cg64(geom, d['x0'], d['rhs'], gamma, k)
             assert rel_l2(x, exact) <= 4 * rel_l2(ref, exact) + 1e-5, (gamma, k, err, rel_l2(x, exact), rel_l2(ref, exact))
     assert torch.equal(x0, torch.from_numpy(d['x0']).cuda())        # start value untouched
 
