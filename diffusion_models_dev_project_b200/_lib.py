@@ -31,6 +31,7 @@ class GeomDesc(C.Structure):
 _F = C.c_void_p   # device float*
 SIGNATURES = {
     "scd_geom_create": (C.c_int, [C.POINTER(GeomDesc), C.POINTER(C.c_void_p)]),
+    "scd_geom_create_weighted": (C.c_int, [C.POINTER(GeomDesc), C.POINTER(C.c_double), C.POINTER(C.c_void_p)]),
     "scd_geom_destroy": (C.c_int, [C.c_void_p]),
     "scd_fp_scratch_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
     "scd_fp": (C.c_int, [C.c_void_p, _F, _F, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),

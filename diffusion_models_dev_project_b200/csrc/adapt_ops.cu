@@ -434,7 +434,9 @@ extern "C" int scd_adapt_bwd(const scd_geom_t *g, const float *grad_loss, const 
     e.c_acc = (float)(2.0 / n_res * trafo_grad_scale);                   // trafo_grad_scale = adj_scale / c_w
     e.add1 = tvg; e.c1 = (float)tv_lambda; e.add2 = nullptr; e.c2 = 0.f;
     e.out2 = nullptr; e.dot_part = nullptr; e.dot_stride = 0; e.dot_with_add1 = 0;
-    if ((rc = scd_launch_bp(g, res, gx, batch, 0, g->n_angles, e, c.w + L.off_q, scd_sino_il_bytes(g, batch), c.st))) return rc;
+    // the transpose of A carries no view weights (a weighted geometry weights A* only)
+    if ((rc = scd_launch_bp(g, res, gx, batch, 0, g->n_angles, e, c.w + L.off_q, scd_sino_il_bytes(g, batch), c.st,
+                            false))) return rc;
     const float *gfinal = gx;                                            // d loss / d xhat0
     if (dc_type == 1) {
         // xhat = xhat0 - gamma A*(A xhat0) + const: adjoint gx - gamma A*(A gx)

@@ -51,11 +51,12 @@ struct BqParams {
 };
 
 // ------------------------------------------------------------ sino pack ---
-// user sinogram [B][n_angles][n_det] -> sino_il (angles [lo,hi) only)
+// user sinogram [B][n_angles][n_det] -> sino_il (angles [lo,hi) only), times the view weight w[a] of A* when
+// w != NULL
 // grid = (bin chunks of 256, angles in range, groups)
 __global__ void __launch_bounds__(256)
 sino_pack_kernel(const float *sino, float *sino_il, int n_angles, int n_det, int batch,
-                 int angle_lo, int SB, int PADL, int NB, size_t group_floats)
+                 int angle_lo, int SB, int PADL, int NB, size_t group_floats, const float *w)
 {
     __shared__ float tile[16][257];
     scd_pdl_wait();                               // predecessor complete, its writes visible
@@ -63,12 +64,13 @@ sino_pack_kernel(const float *sino, float *sino_il, int n_angles, int n_det, int
     const int tid = threadIdx.x;
     const int J0 = blockIdx.x * 256, a = angle_lo + blockIdx.y, grp = blockIdx.z;
     const int j = J0 + tid;
+    const float wa = w ? __ldg(w + a) : 1.f;
     for (int s = 0; s < SB; ++s) {
         const int b = grp * SB + s;
         float v = 0.f;
         if (b < batch && j >= PADL && j < PADL + n_det)
             v = __ldg(sino + ((size_t)b * n_angles + a) * n_det + (j - PADL));
-        tile[s][tid] = v;
+        tile[s][tid] = w ? v * wa : v;
     }
     __syncthreads();
     float *dst = sino_il + (size_t)grp * group_floats + ((size_t)a * NB + J0) * SB;
@@ -652,15 +654,16 @@ int scd_launch_bp_il(const scd_geom *g, const float *sino_il, float *out, int ba
 }
 
 int scd_launch_sino_pack(const scd_geom *g, const float *sino, float *sino_il, int batch,
-                         int angle_lo, int angle_hi, cudaStream_t st)
+                         int angle_lo, int angle_hi, cudaStream_t st, bool weighted)
 {
     if (batch <= 0 || angle_hi <= angle_lo) return 0;
     const int SB = scd_group_samples(g, batch);
     const int groups = (batch + SB - 1) / SB;
     dim3 grid((g->il_nb + 255) / 256, angle_hi - angle_lo, groups);
     if (grid.y > 65535 || grid.z > 65535) { scd_set_error("scd_bp: too many angles / samples"); return SCD_E_INVALID; }
+    const float *w = weighted ? g->d_w : nullptr;
     SCD_CUDA(scd_launch_kernel(sino_pack_kernel, grid, dim3(256), 0, st, 0, sino, sino_il, g->n_angles, g->n_det, batch,
-                               angle_lo, SB, g->il_padl, g->il_nb, (size_t)g->n_angles * g->il_nb * SB));
+                               angle_lo, SB, g->il_padl, g->il_nb, (size_t)g->n_angles * g->il_nb * SB, w));
     SCD_LAUNCH_CHECK("sino_pack_kernel");
     return 0;
 }
@@ -668,7 +671,7 @@ int scd_launch_sino_pack(const scd_geom *g, const float *sino, float *sino_il, i
 // ----------------------------------------------------- user-layout entry ---
 int scd_launch_bp(const scd_geom *g, const float *sino, float *out, int batch,
                   int angle_lo, int angle_hi, const BpEpilogue &ep, void *scratch, size_t scratch_bytes,
-                  cudaStream_t st)
+                  cudaStream_t st, bool weighted)
 {
     if (g && batch == 0) return 0;                 // empty batch: nothing to do (pointers may be null)
     if (!g || !sino || (!out && !ep.n_bands)) { scd_set_error("scd_bp: null argument"); return SCD_E_INVALID; }
@@ -685,7 +688,7 @@ int scd_launch_bp(const scd_geom *g, const float *sino, float *out, int batch,
                       scratch_bytes, need + 256);
         return SCD_E_WORKSPACE;
     }
-    int rc = scd_launch_sino_pack(g, sino, (float *)sp, batch, angle_lo, angle_hi, st);
+    int rc = scd_launch_sino_pack(g, sino, (float *)sp, batch, angle_lo, angle_hi, st, weighted);
     if (rc) return rc;
     return scd_launch_bp_il(g, (const float *)sp, out, batch, angle_lo, angle_hi, ep, st);
 }

@@ -72,6 +72,7 @@ struct MqParams {
     const FpAngle *fp;
     const float2  *rayt;     // [order position][n_det] (u0 + 1, b) per ray
     const float2  *angt;     // [order position] (scale, angle id bits)
+    const float   *angw;     // [order position] view weight of the interleaved output (A* quadrature) or NULL
     const int     *order;
     int n0, n1, n_angles, n_det, batch;
     int NA;                  // largest number of angles per CTA (sizes the tables)
@@ -666,7 +667,8 @@ fp_march_kernel(const MqParams P, const __grid_constant__ CUtensorMap tm0, const
                 for (int v = 0; v < V; ++v) sum[v] += pf[v];
             }
             const int ai = e / n_det, j = e - ai * n_det;
-            const float sc = ang[ai].scale;
+            // the view weight of A* rides on the output scale: linear, so the recurrence below stays exact
+            const float sc = P.angw ? ang[ai].scale * __ldg(P.angw + pos0 + ai) : ang[ai].scale;
             VT ov;
             float *of = reinterpret_cast<float *>(&ov);
 #pragma unroll
@@ -1099,7 +1101,7 @@ static void mq_fill_params(const scd_geom *g, const MqConfig &c, MqParams &P, fl
 {
     memset(&P, 0, sizeof(P));
     P.sino = sino; P.sino_il = sino_il; P.il_padl = g->il_padl; P.il_nb = g->il_nb;
-    P.fp = g->d_fp; P.rayt = g->d_rayt; P.angt = g->d_angt; P.order = g->d_order;
+    P.fp = g->d_fp; P.rayt = g->d_rayt; P.angt = g->d_angt; P.angw = g->d_angw; P.order = g->d_order;
     P.n0 = g->n0; P.n1 = g->n1; P.n_angles = g->n_angles; P.n_det = g->n_det; P.batch = batch;
     P.NA = c.NA; P.nbuf = c.nbuf; P.CS = c.CS; P.rows_per_cta = c.rows_per_cta; P.ring_bytes = (int)c.ring_bytes; P.L = c.L;
     P.need_cls[0] = ncls[0] > 0; P.need_cls[1] = ncls[1] > 0;

@@ -56,8 +56,24 @@ extern "C" void scd_launch_count_reset(void) { g_launches.store(0, std::memory_o
 
 extern "C" int scd_geom_create(const scd_geom_desc *d, scd_geom_t **out)
 {
+    return scd_geom_create_weighted(d, nullptr, out);
+}
+
+extern "C" int scd_geom_create_weighted(const scd_geom_desc *d, const double *wts, scd_geom_t **out)
+{
     if (!d || !out) { scd_set_error("scd_geom_create: null argument"); return SCD_E_INVALID; }
     *out = nullptr;
+    if (wts && d->n_angles >= 1) {
+        bool all_one = true;
+        for (int i = 0; i < d->n_angles; ++i) {
+            if (!std::isfinite(wts[i]) || !(wts[i] > 0.0)) {
+                scd_set_error("scd_geom_create_weighted: angle weight %d is %g (must be finite and > 0)", i, wts[i]);
+                return SCD_E_INVALID;
+            }
+            all_one = all_one && wts[i] == 1.0;
+        }
+        if (all_one) wts = nullptr;               // the unweighted geometry: no table, the same launches
+    }
     if (d->n0 < 1 || d->n1 < 1 || d->n_angles < 1 || d->n_det < 2 || !d->angles ||
         !(d->dx > 0) || !(d->ds > 0)) {
         scd_set_error("scd_geom_create: invalid geometry (n0=%d n1=%d n_angles=%d n_det=%d dx=%g ds=%g)",
@@ -172,6 +188,18 @@ extern "C" int scd_geom_create(const scd_geom_desc *d, scd_geom_t **out)
         scd_geom_destroy(g);
         return scd_cuda_fail(ce, "scd_geom_create upload");
     }
+    if (wts) {
+        std::vector<float> w_pos((size_t)na), w_id((size_t)na);
+        for (int p = 0; p < na; ++p) w_pos[p] = (float)wts[g->h_order[p]];
+        for (int i = 0; i < na; ++i) w_id[i] = (float)wts[i];
+        if ((ce = cudaMalloc(&g->d_angw, sizeof(float) * na)) != cudaSuccess ||
+            (ce = cudaMemcpy(g->d_angw, w_pos.data(), sizeof(float) * na, cudaMemcpyHostToDevice)) != cudaSuccess ||
+            (ce = cudaMalloc(&g->d_w, sizeof(float) * na)) != cudaSuccess ||
+            (ce = cudaMemcpy(g->d_w, w_id.data(), sizeof(float) * na, cudaMemcpyHostToDevice)) != cudaSuccess) {
+            scd_geom_destroy(g);
+            return scd_cuda_fail(ce, "scd_geom_create_weighted upload");
+        }
+    }
     *out = g;
     return 0;
 }
@@ -185,6 +213,8 @@ extern "C" int scd_geom_destroy(scd_geom_t *g)
     if (g->d_rayt) cudaFree(g->d_rayt);
     if (g->d_angt) cudaFree(g->d_angt);
     if (g->d_zero_row) cudaFree(g->d_zero_row);
+    if (g->d_angw) cudaFree(g->d_angw);
+    if (g->d_w) cudaFree(g->d_w);
     free(g->h_fp); free(g->h_bp); free(g->h_order);
     free(g);
     return 0;

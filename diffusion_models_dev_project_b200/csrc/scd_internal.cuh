@@ -127,6 +127,10 @@ struct scd_geom {
     float2  *d_rayt;      // [n_angles][n_det] (u0 + 1, b): start position (row 0) and slope of every ray, from fp64;
                           // rows in order[] order (position p holds angle order[p])
     float2  *d_angt;      // [n_angles] (scale, id as int bits) in order[] order
+    // view weights (scd_geom_create_weighted), NULL when every view weighs 1: applied to the interleaved sinogram
+    // the backprojector reads, never to A's user-layout output
+    float   *d_angw;      // [n_angles] w_i in order[] order (projector output)
+    float   *d_w;         // [n_angles] w_i by angle id (sinogram re-layout)
     float   *d_zero_row;  // max(n0, n1) * 16 zero floats: source of projector strip rows beyond the image
     // host copies
     FpAngle *h_fp;
@@ -227,10 +231,11 @@ struct BpEpilogue {
     int il = 0, mode = 0;
     const float *beta = nullptr;
 };
-// sino in user layout; scratch (>= scd_sino_il_bytes) receives the interleaved copy
+// sino in user layout; scratch (>= scd_sino_il_bytes) receives the interleaved copy, times the view weights unless
+// weighted == false (the plain transpose of A, gradient of the adaptation objective)
 int scd_launch_bp(const scd_geom *g, const float *sino, float *out, int batch,
                   int angle_lo, int angle_hi, const BpEpilogue &ep, void *scratch, size_t scratch_bytes,
-                  cudaStream_t st);
+                  cudaStream_t st, bool weighted = true);
 int scd_launch_bp_il(const scd_geom *g, const float *sino_il, float *out, int batch,
                      int angle_lo, int angle_hi, const BpEpilogue &ep, cudaStream_t st);
 // banded stores + rank-ordered reduction of the bands (peer_reduce.cu)
@@ -238,7 +243,7 @@ int scd_launch_band_reduce(const float *stage, int n_src, int64_t slot_stride, i
                            int n1, int row_lo, int n0, float *const *out_ptrs, int n_out, int multicast,
                            const float *addend, float c_add, float c_sum, cudaStream_t st);
 int scd_launch_sino_pack(const scd_geom *g, const float *sino, float *sino_il, int batch,
-                         int angle_lo, int angle_hi, cudaStream_t st);
+                         int angle_lo, int angle_hi, cudaStream_t st, bool weighted = true);
 size_t scd_sino_il_bytes(const scd_geom *g, int batch);
 // number of dot_part entries per sample the BP launch for this batch writes (current tuning) /
 // an upper bound independent of the tuning (workspace sizing)

@@ -39,7 +39,14 @@ class _GeomHandle:
             n_det=geom.n_det, s_min=geom.s_min, ds=geom.ds, adj_scale=adj_scale)
         h = C.c_void_p()
         with torch.cuda.device(device):
-            _lib.check(lib.scd_geom_create(C.byref(desc), C.byref(h)), 'scd_geom_create')
+            if geom.angle_weights is None:
+                _lib.check(lib.scd_geom_create(C.byref(desc), C.byref(h)), 'scd_geom_create')
+            else:
+                w = np.ascontiguousarray(geom.angle_weights, dtype=np.float64)
+                if w.shape != (geom.n_angles,):
+                    raise ValueError('angle_weights: expected shape (%d,), got %r' % (geom.n_angles, w.shape))
+                _lib.check(lib.scd_geom_create_weighted(C.byref(desc), w.ctypes.data_as(C.POINTER(C.c_double)),
+                                                        C.byref(h)), 'scd_geom_create_weighted')
         self.ptr = h
         self.device = device
         self._lib = lib
@@ -55,7 +62,8 @@ class _GeomHandle:
 
 class _TrafoFn(torch.autograd.Function):
     """y = A x.  Backward: the unweighted transpose A^T g = A*(g)/c_w (ODL
-    ``OperatorFunction`` convention, SURVEY.md §8b)."""
+    ``OperatorFunction`` convention, SURVEY.md §8b).  With view weights w_i, A* carries them and the
+    transpose is A*(g / w)/c_w (c_w: the mean cell)."""
 
     @staticmethod
     def forward(ctx, x, rt):
@@ -65,11 +73,14 @@ class _TrafoFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         rt = ctx.rt
+        w = rt._view_weights(g.device)
+        if w is not None:
+            g = g / w
         return _AdjointFn.apply(g, rt) * (1.0 / rt.geometry.range_weight), None
 
 
 class _AdjointFn(torch.autograd.Function):
-    """x = A* y.  Backward: c_w * A g."""
+    """x = A* y.  Backward: c_i * (A g)_i with the per-view cell c_i = c_w * w_i."""
 
     @staticmethod
     def forward(ctx, y, rt):
@@ -79,7 +90,9 @@ class _AdjointFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         rt = ctx.rt
-        return _TrafoFn.apply(g, rt) * rt.geometry.range_weight, None
+        ag = _TrafoFn.apply(g, rt) * rt.geometry.range_weight
+        w = rt._view_weights(g.device)
+        return (ag if w is None else ag * w), None
 
 
 class NormalOp:
@@ -111,17 +124,30 @@ class B200RayTrafo(BaseRayTrafo):
         ``'b200'`` (or the reference's ``'odl'`` / ``'iradon'`` names, which
         select the same kernels -- there is exactly one implementation).
     adjoint_scaling : {'dphi', 'dphi/ds'}
-        ``A* = adj_scale * sum_i lerp(y[i], t_i(x))``; ``'dphi'`` (default) is the
+        ``A* = adj_scale * sum_i w_i lerp(y[i], t_i(x))``; ``'dphi'`` (default) is the
         continuous weighted adjoint (kappa = 1 of SURVEY.md §8c), ``'dphi/ds'``
-        the alternative kappa = 1/ds convention.
+        the alternative kappa = 1/ds convention.  ``dphi`` is the mean angle cell and
+        ``w_i`` the view weights of the geometry (1 for a uniform partition).
+    geometry : ParallelBeamGeometry2D, optional
+        An explicit geometry (angle list and view weights, detector partition, pixel size,
+        domain offset) instead of the one ``SimpleTrafo`` derives from ``(im_shape, num_angles)``;
+        e.g. ``ParallelBeamGeometry2D.from_angles`` for golden-angle or randomly dropped views.
+    angle_range : (float, float), optional
+        ``num_angles`` cell-centred views on ``[min, max)`` radians instead of ``[0, pi)``: the
+        limited-angle (missing wedge) geometry of ``ParallelBeamGeometry2D.from_angle_range``.
     """
 
-    def __init__(self, im_shape, num_angles, impl='b200', adjoint_scaling='dphi', geometry=None):
+    def __init__(self, im_shape, num_angles, impl='b200', adjoint_scaling='dphi', geometry=None, angle_range=None):
         if impl not in ('b200', 'odl', 'iradon'):
             raise NotImplementedError(impl)
-        # `geometry`: an explicit ParallelBeamGeometry2D (arbitrary angle list, detector partition, pixel
-        # size, domain offset) instead of the one SimpleTrafo derives from (im_shape, num_angles)
-        geom = geometry if geometry is not None else ParallelBeamGeometry2D.from_im_shape(im_shape, num_angles)
+        if geometry is not None and angle_range is not None:
+            raise ValueError('pass either geometry or angle_range')
+        if geometry is not None:
+            geom = geometry
+        elif angle_range is not None:
+            geom = ParallelBeamGeometry2D.from_angle_range(im_shape, num_angles, *angle_range)
+        else:
+            geom = ParallelBeamGeometry2D.from_im_shape(im_shape, num_angles)
         if geometry is not None and (tuple(im_shape) != geom.im_shape or int(num_angles) != geom.n_angles):
             raise ValueError('geometry does not match im_shape / num_angles')
         super().__init__(im_shape=tuple(int(v) for v in im_shape), obs_shape=geom.obs_shape)
@@ -135,6 +161,7 @@ class B200RayTrafo(BaseRayTrafo):
         self._angles = geom.angles
         self._handles = {}
         self._work = {}
+        self._weights = {}
         self._hlock = threading.Lock()
 
     # ------------------------------------------------------------ plumbing ---
@@ -155,6 +182,16 @@ class B200RayTrafo(BaseRayTrafo):
                     h = _GeomHandle(self.geometry, self.adj_scale, torch.device('cuda', idx))
                     self._handles[idx] = h
         return h
+
+    def _view_weights(self, device):
+        """The view weights as a float32 ``[n_angles, 1]`` tensor on ``device`` (cached), or None if uniform."""
+        if self.geometry.angle_weights is None:
+            return None
+        w = self._weights.get(device)
+        if w is None:
+            w = torch.as_tensor(self.geometry.view_weights, dtype=torch.float32, device=device).reshape(-1, 1)
+            self._weights[device] = w
+        return w
 
     def set_tuning(self, device, **kw):
         """Override launch heuristics (see scd_set_tuning)."""
@@ -513,5 +550,10 @@ class B200RayTrafo(BaseRayTrafo):
         of two >= 2 N_s, "ramp" Fourier filter ``2 Re FFT(f)`` of the Kak-Slaney kernel, scale
         ``pi/(2 N_theta)``), evaluated as the equivalent linear convolution by ``scd_ramp_filter``; the
         recipe's constants are split as ``2 * pi/(2 N_theta) = dphi`` (the weight of the pixel-driven
-        backprojector) times ``1/ds`` (the recipe assumes a unit detector cell; ours is ``ds``)."""
+        backprojector) times ``1/ds`` (the recipe assumes a unit detector cell; ours is ``ds``).
+
+        On a weighted geometry the backprojector sums view ``i`` with ``dphi * w_i``, its angular cell: the
+        FBP quadrature of a non-uniform view set.  On a wedge the result is the truncated FBP -- the inverse
+        Radon formula restricted to the measured angles -- not a limited-angle reconstruction: the missing
+        wedge stays missing (streaks and lost edges along it)."""
         return self._bp(self.ramp_filter(observation), self.geometry.dphi)

@@ -55,8 +55,11 @@ class _AdaptationLossFn(torch.autograd.Function):
         with torch.cuda.device(dev):
             _lib.check(lib.scd_tv_grad(x.data_ptr(), tvg.data_ptr(), ctx.images, rt.im_shape[0], rt.im_shape[1], stream),
                        'scd_tv_grad')
+        # the gradient of the residual is the plain transpose of A: adj_scale/c_w = dx^2/ds times the unweighted
+        # backprojection sum, so the view weights that scd_bp applies for A* are divided out first
         scale = 2.0 / ctx.numel * rt.adj_scale / rt.geometry.range_weight
-        grad = rt._bp(r, scale, addend=tvg, addend_scale=ctx.lam)
+        w = rt._view_weights(dev)
+        grad = rt._bp(r if w is None else r / w, scale, addend=tvg, addend_scale=ctx.lam)
         return grad * g, None, None, None
 
 
@@ -141,6 +144,7 @@ class _AdaptObjectiveFn(torch.autograd.Function):
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         with torch.cuda.device(dev):
             _lib.check(lib.scd_adapt_bwd(h.ptr, g.data_ptr(), ctx.t.data_ptr(), ctx.abar.data_ptr(), int(ctx.abar.numel()),
+                                         # dx^2/ds: the mean cell cancels; the call backprojects without view weights
                                          gamma, n_iter, dc_code, lam, rt.adj_scale / rt.geometry.range_weight,
                                          grad_s.data_ptr(), ctx.batch, ctx.wp, ctx.n_work, stream), 'scd_adapt_bwd')
         ctx.work = None

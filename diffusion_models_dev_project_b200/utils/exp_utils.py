@@ -2,7 +2,9 @@
 
 ``get_standard_ray_trafo(config)`` returns the CUDA-kernel operator for
 ``trafo_name='simple_trafo'`` whatever ``forward_op.impl`` says (there is one
-implementation).  ``get_standard_sampler`` keeps the reference's signature but
+implementation); the optional keys ``forward_op.angle_range`` (a limited-angle wedge)
+and ``forward_op.angles`` (an explicit, possibly non-uniform view set) select other
+angle sets.  ``get_standard_sampler`` keeps the reference's signature but
 builds the DDPM/'dds' sampler correctly: the reference passes an
 ``init_chain_fn`` keyword ``BaseSampler`` does not accept and therefore raises
 (exp_utils.py:214-221, see SURVEY.md §3.1); only the branch the hot path needs
@@ -15,6 +17,7 @@ import torch
 
 from .sde import VESDE, VPSDE, DDPM, _EPSILON_PRED_CLASSES
 from ..physics import B200RayTrafo, simulate
+from ..physics.geometry import ParallelBeamGeometry2D
 from ..samplers import (BaseSampler, decomposed_diffusion_sampling_sde_predictor,
                         adapted_ddim_sde_predictor, tv_loss, adaptation_loss, AdaptationLoss, _adapt, _score_model_adpt,
                         Euler_Maruyama_sde_predictor, Ancestral_Sampling)
@@ -31,11 +34,37 @@ def get_standard_sde(config):
     raise NotImplementedError(name)
 
 
+def _optional(ns, key):
+    """``ns.key`` or None: config objects signal a missing key with AttributeError (namespaces, ConfigDict) or
+    KeyError (dicts with attribute access)."""
+    try:
+        return getattr(ns, key)
+    except (AttributeError, KeyError):
+        return None
+
+
 def get_standard_ray_trafo(config):
-    if config.forward_op.trafo_name.lower() == 'simple_trafo':
-        return B200RayTrafo(im_shape=(config.data.im_size, config.data.im_size),
-                            num_angles=config.forward_op.num_angles, impl=config.forward_op.impl)
-    raise NotImplementedError(config.forward_op.trafo_name)
+    """``forward_op.angle_range = (min, max)`` (radians): ``num_angles`` cell-centred views on ``[min, max)``.
+    ``forward_op.angles`` (radians): exactly these views, weighted by their angular cells (``num_angles`` may be
+    omitted; if given it must equal their count).  Without either key: ``num_angles`` views on ``[0, pi)``."""
+    fo = config.forward_op
+    if fo.trafo_name.lower() != 'simple_trafo':
+        raise NotImplementedError(fo.trafo_name)
+    im_shape = (config.data.im_size, config.data.im_size)
+    angle_range = _optional(fo, 'angle_range')
+    angles = _optional(fo, 'angles')
+    if angle_range is not None and angles is not None:
+        raise ValueError('forward_op: give angle_range or angles, not both')
+    if angles is not None:
+        geom = ParallelBeamGeometry2D.from_angles(im_shape, angles)
+        num_angles = _optional(fo, 'num_angles')
+        if num_angles is not None and int(num_angles) != geom.n_angles:
+            raise ValueError('forward_op.num_angles = %d but %d angles are given' % (int(num_angles), geom.n_angles))
+        return B200RayTrafo(im_shape=im_shape, num_angles=geom.n_angles, impl=fo.impl, geometry=geom)
+    if angle_range is not None:
+        return B200RayTrafo(im_shape=im_shape, num_angles=fo.num_angles, impl=fo.impl,
+                            angle_range=tuple(float(a) for a in angle_range))
+    return B200RayTrafo(im_shape=im_shape, num_angles=fo.num_angles, impl=fo.impl)
 
 
 def get_data_from_ground_truth(ground_truth, ray_trafo, white_noise_rel_stddev):

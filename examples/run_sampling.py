@@ -9,6 +9,8 @@ data-consistency path, not a trained prior), a small LoRA injector instead of th
 
     python examples/run_sampling.py --mode conditional --method dds --num_steps 20
     python examples/run_sampling.py --mode adapted --num_steps 10 --num_optim_step 2 --add_cg
+    python examples/run_sampling.py --num_steps 20 --angle_range 0 90        # limited angle: a 90 degree wedge
+    python examples/run_sampling.py --num_steps 20 --angles_file views.txt   # sparse / non-uniform views
 """
 import argparse
 import os
@@ -54,6 +56,11 @@ def parse():
     # synthetic set-up
     p.add_argument('--im_size', type=int, default=256)
     p.add_argument('--num_angles', type=int, default=60)
+    p.add_argument('--angle_range', type=float, nargs=2, default=None, metavar=('MIN', 'MAX'),
+                   help='limited angle: num_angles cell-centred views on [MIN, MAX) degrees instead of [0, 180)')
+    p.add_argument('--angles_file', default=None,
+                   help='text file of view angles in degrees (whitespace or newline separated), weighted by their '
+                        'angular cells; replaces --num_angles')
     p.add_argument('--batch_size', type=int, default=1)
     p.add_argument('--num_images', type=int, default=1)
     p.add_argument('--unet', default='small', choices=['small', 'aapm', 'blur'],
@@ -66,11 +73,19 @@ def parse():
 def main():
     args = parse()
     device = torch.device('cuda')
+    forward_op = NS(trafo_name='simple_trafo', num_angles=args.num_angles, impl='b200')
+    if args.angle_range is not None and args.angles_file is not None:
+        raise SystemExit('give --angle_range or --angles_file, not both')
+    if args.angle_range is not None:
+        forward_op.angle_range = tuple(np.deg2rad(args.angle_range))
+    if args.angles_file is not None:
+        forward_op.angles = np.deg2rad(np.loadtxt(args.angles_file, dtype=np.float64).reshape(-1))
+        forward_op.num_angles = int(forward_op.angles.size)
     config = NS(
         device=device, seed=args.seed,
         sde=NS(type=args.sde, beta_min=1e-4, beta_max=0.02, num_steps=1000, sigma_min=0.01, sigma_max=50.),
         data=NS(im_size=args.im_size, stddev=float(args.noise_level)),
-        forward_op=NS(trafo_name='simple_trafo', num_angles=args.num_angles, impl='b200'),
+        forward_op=forward_op,
         sampling=NS(batch_size=args.batch_size, eps=1e-3, travel_length=1, travel_repeat=1),
         model=NS(in_channels=1))
     if args.sde != 'ddpm':

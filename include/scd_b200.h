@@ -64,6 +64,17 @@ typedef struct scd_geom_desc {
 /* Build the device-side tables for one geometry on the current device.
  * Replaces: SimpleTrafo.__init__ (src/physics/trafo.py:17-51).              */
 int scd_geom_create(const scd_geom_desc *desc, scd_geom_t **out);
+
+/* Same geometry with a weight per view: A* = adj_scale * sum_i w_i * lerp(sino[i], t_i(x)).
+ * angle_weights[n_angles] is the relative angular cell of each view (ODL's nonuniform_partition /
+ * uniform_partition of a wedge, mean 1; finite and > 0).  It makes A* the quadrature of a
+ * limited-angle or non-uniform view set.  A (scd_fp) stays unweighted.  The weight is applied where the
+ * sinogram the backprojector reads is written: by the projector's interleaved output (scd_fp_il,
+ * scd_fp_ilimg, scd_cg, scd_dds_step, the operator applications of scd_adapt_fwd/bwd) and by the
+ * re-layout of a user sinogram (scd_bp, scd_bp_banded).  The gradient backprojection of
+ * scd_adapt_bwd stays unweighted: it is the transpose of A.
+ * angle_weights == NULL, or every entry exactly 1.0: identical to scd_geom_create.                      */
+int scd_geom_create_weighted(const scd_geom_desc *desc, const double *angle_weights, scd_geom_t **out);
 int scd_geom_destroy(scd_geom_t *g);
 
 /* A: forward projection of angles [angle_lo, angle_hi) (rows outside that
