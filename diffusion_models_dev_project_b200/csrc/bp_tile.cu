@@ -603,20 +603,28 @@ static int bq_launch_t(const BqParams &P, const BqConfig &c, cudaStream_t st, in
     return 0;
 }
 
+// banded output: every tile lies inside one band and every band has somewhere to go
+static int bq_check_bands(const scd_geom *g, const BpEpilogue &ep)
+{
+    if (ep.n_bands > SCD_MAX_BANDS || ep.band_rows <= 0 || ep.band_rows % 32 != 0 ||
+        (long)ep.n_bands * ep.band_rows < g->n0) {
+        scd_set_error("scd_bp: bad band layout (%d bands of %d rows for %d image rows; rows must be a multiple of 32)",
+                      ep.n_bands, ep.band_rows, g->n0);
+        return SCD_E_INVALID;
+    }
+    for (int i = 0; i < ep.n_bands; ++i)
+        if (!ep.band_out[i]) { scd_set_error("scd_bp: null band pointer"); return SCD_E_INVALID; }
+    return 0;
+}
+
 int scd_launch_bp_il(const scd_geom *g, const float *sino_il, float *out, int batch,
                      int angle_lo, int angle_hi, const BpEpilogue &ep, cudaStream_t st)
 {
     if (!g || !sino_il || (!out && !ep.n_bands)) { scd_set_error("scd_bp: null argument"); return SCD_E_INVALID; }
     if (batch <= 0) return 0;
     if (ep.n_bands) {
-        if (ep.n_bands > SCD_MAX_BANDS || ep.band_rows <= 0 || ep.band_rows % 32 != 0 ||
-            (long)ep.n_bands * ep.band_rows < g->n0) {
-            scd_set_error("scd_bp: bad band layout (%d bands of %d rows for %d image rows; rows must be a multiple of 32)",
-                          ep.n_bands, ep.band_rows, g->n0);
-            return SCD_E_INVALID;
-        }
-        for (int i = 0; i < ep.n_bands; ++i)
-            if (!ep.band_out[i]) { scd_set_error("scd_bp: null band pointer"); return SCD_E_INVALID; }
+        const int rc = bq_check_bands(g, ep);
+        if (rc) return rc;
     }
     BqConfig c = bq_choose(g, batch, angle_lo, angle_hi);
     if (ep.n_bands && c.th_eff != c.TH) {          // bands are aligned to whole tiles
@@ -681,6 +689,10 @@ int scd_launch_bp(const scd_geom *g, const float *sino, float *out, int batch,
         return SCD_E_INVALID;
     }
     if (batch == 0) return 0;
+    if (ep.n_bands) {                              // before the re-layout: a rejected call writes nothing
+        const int rc = bq_check_bands(g, ep);
+        if (rc) return rc;
+    }
     const uintptr_t sp = ((uintptr_t)scratch + 127) & ~(uintptr_t)127;
     const size_t need = scd_sino_il_bytes(g, batch) - 256;
     if (!scratch || sp + need > (uintptr_t)scratch + scratch_bytes) {
