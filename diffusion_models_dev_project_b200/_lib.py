@@ -15,6 +15,8 @@ SCD_E_INVALID = -10001
 SCD_E_NODEVICE = -10002
 SCD_E_WORKSPACE = -10003
 
+SCD_GEOM_MATCHED_ADJOINT = 0x1     # scd_geom_create_ex flag: A* is the exact transpose of A
+
 
 class GeomDesc(C.Structure):
     _fields_ = [
@@ -32,6 +34,7 @@ _F = C.c_void_p   # device float*
 SIGNATURES = {
     "scd_geom_create": (C.c_int, [C.POINTER(GeomDesc), C.POINTER(C.c_void_p)]),
     "scd_geom_create_weighted": (C.c_int, [C.POINTER(GeomDesc), C.POINTER(C.c_double), C.POINTER(C.c_void_p)]),
+    "scd_geom_create_ex": (C.c_int, [C.POINTER(GeomDesc), C.POINTER(C.c_double), C.c_uint32, C.POINTER(C.c_void_p)]),
     "scd_geom_destroy": (C.c_int, [C.c_void_p]),
     "scd_fp_scratch_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
     "scd_fp": (C.c_int, [C.c_void_p, _F, _F, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -23,6 +23,13 @@
 //   thread  = PPT pixels in a column (k0 .. k0+PPT-1), accumulators in registers
 //   angle range [lo,hi): the angle-sharded variant (multi-GPU config 4) is the same kernel;
 //             partial images are summed by the caller (NCCL).
+//
+// Matched adjoint (MT = true, geometries created with SCD_GEOM_MATCHED_ADJOINT): the exact transpose of the
+// Joseph projector, c_w * J^T y = dphi * sum_i w_i sum_j k_i max(0, 1 - k_i |j - v|) y_ij with
+// k_i = 1 / max(|ci|, |si|) -- the same march with the unit hat (1-f, f) replaced by a hat of unit area and
+// half-width h_i = 1/k_i <= dx/ds < 1.5.  Views with h_i <= 1 keep the two taps floor(v), floor(v)+1 (and the
+// pair march); the few near-axis views with h_i > 1 take three taps around round(v).  k_i and the 2/3-tap
+// choice are derived per view from (ci, si) of the shared-memory table: warp-uniform.
 #include "scd_internal.cuh"
 #include <algorithm>
 #include <cmath>
@@ -179,12 +186,23 @@ __device__ __forceinline__ void bq_tap3(float (&p)[4], float4 t0, float4 t1, flo
     p[0] = a.x; p[1] = a.y; p[2] = b.x; p[3] = b.y;
 }
 
+// Matched adjoint: the normalised hat k * max(0, 1 - k*d) at distance d from the pixel's detector coordinate
+__device__ __forceinline__ float bq_hat(float k, float d) { return k * fmaxf(0.0f, fmaf(-k, d, 1.0f)); }
+
+// Weights of the two taps floor(z), floor(z)+1 at fraction w = z - floor(z): (1-w, w), or the normalised hat (MT)
+template <bool MT>
+__device__ __forceinline__ void bq_w2(float k, float w, float &wl, float &wr)
+{
+    if (MT) { wl = bq_hat(k, w); wr = bq_hat(k, 1.0f - w); }
+    else    { wl = 1.0f - w; wr = w; (void)k; }
+}
+
 // Pair march of two pixels of a column whose detector coordinates satisfy zlo <= zhi < zlo + 1: their four taps lie
 // in the three consecutive bins starting at floor(zlo) -- 3 loads instead of 4.  The lower pixel takes (1-w, w) on bins
 // 0, 1; the upper one (1-w, w, 0) or (0, 1-w, w).  The product with the exact zero changes nothing and the real taps
-// are added in the order of the plain march: bit-identical to it.
-template <int V, int SB>
-__device__ __forceinline__ void bq_pair(float (&acc_lo)[V], float (&acc_hi)[V], float zlo, float zhi, unsigned seg)
+// are added in the order of the plain march: bit-identical to it.  MT: the same with the two hat weights of bq_w2.
+template <int V, int SB, bool MT>
+__device__ __forceinline__ void bq_pair(float (&acc_lo)[V], float (&acc_hi)[V], float zlo, float zhi, unsigned seg, float k)
 {
     typedef BqVec<V> LD;
     typedef typename LD::T VT;
@@ -195,15 +213,17 @@ __device__ __forceinline__ void bq_pair(float (&acc_lo)[V], float (&acc_hi)[V], 
     const VT b0 = LD::template ld<0>(ad);
     const VT b1 = LD::template ld<SB * 4>(ad);
     const VT b2 = LD::template ld<2 * SB * 4>(ad);
-    bq_tap(acc_lo, b0, b1, 1.0f - wlo, wlo);
+    float ll, lr, ul, ur;
+    bq_w2<MT>(k, wlo, ll, lr);
+    bq_tap(acc_lo, b0, b1, ll, lr);
     const bool s = ihi != ilo;                                   // the upper pixel's left tap is bin 1
-    const float uh = 1.0f - whi;
-    bq_tap3(acc_hi, b0, b1, b2, s ? 0.0f : uh, s ? uh : whi, s ? whi : 0.0f);
+    bq_w2<MT>(k, whi, ul, ur);
+    bq_tap3(acc_hi, b0, b1, b2, s ? 0.0f : ul, s ? ul : ur, s ? ur : 0.0f);
 }
 
 // V samples per lane, LPR lanes per pixel (SB = V*LPR), PPT pixels per thread; IL: the epilogue's images are
-// sample-interleaved (il images)
-template <int V, int LPR, int PPT, bool IL>
+// sample-interleaved (il images); MT: matched adjoint (exact transpose of the Joseph projector)
+template <int V, int LPR, int PPT, bool IL, bool MT = false>
 __global__ void __launch_bounds__(BQ_THREADS, 2)
 bp_tile_kernel(const BqParams P)
 {
@@ -267,8 +287,9 @@ bp_tile_kernel(const BqParams P)
     const int k0b = K0 + wy * PPT;
 
     // The epilogue's addends are fetched before the march so that their latency hides behind it
-    // (when they fit in a few registers; taller tiles load them in the epilogue).
-    constexpr bool PREF = PPT * V <= 8;
+    // (when they fit in a few registers; taller tiles load them in the epilogue, and so does the matched march,
+    // whose extra weights would otherwise push the prefetched addends into local memory).
+    constexpr bool PREF = PPT * V <= 8 && !MT;
     float pa1[PREF ? PPT : 1][V], pa2[PREF ? PPT : 1][V];
     if (IL) {
         if (PREF && warp < BQ_NW) {
@@ -341,6 +362,27 @@ bp_tile_kernel(const BqParams P)
             for (int i = 0; i < nac; ++i, seg += SEGB, ca += 16u) {
                 const float4 cs = BqVec<4>::ld<0>(ca);
                 const float vb = fmaf(lxf, cs.y, cs.z);
+                float k = 1.0f;
+                if (MT) {
+                    const float h = fmaxf(fabsf(cs.x), fabsf(cs.y));     // half-width of the hat, < 1.5 bins
+                    k = __fdividef(1.0f, h);
+                    if (h > 1.0f) {
+                        // near-axis view: three taps round(z)-1 .. round(z)+1 at distances 1+f, |f|, 1-f
+                        // (f = z - round(z) in [-1/2, 1/2]); round(z)+-2 lie >= 1.5 > h away
+#pragma unroll
+                        for (int m = 0; m < PPT; ++m) {
+                            const float z = fmaf(kyf[m], cs.x, vb);
+                            const float t = __fadd_rd(z + 0.5f, BQ_MAGIC);  // round(z) in the mantissa (z >= 1)
+                            const float f = z - (t - BQ_MAGIC);
+                            const unsigned ad = seg + (unsigned)(__float_as_int(t) - 1) * (unsigned)(SB * 4);
+                            const VT t0 = LD::template ld<0>(ad);
+                            const VT t1 = LD::template ld<SB * 4>(ad);
+                            const VT t2 = LD::template ld<2 * SB * 4>(ad);
+                            bq_tap3(acc[m], t0, t1, t2, bq_hat(k, 1.0f + f), bq_hat(k, fabsf(f)), bq_hat(k, 1.0f - f));
+                        }
+                        continue;
+                    }
+                }
                 if (PPT >= 2 && share_taps && fabsf(cs.x) <= 0.999f) {
                     // Pair march: the two pixels of a column pair are |ci| < 1 bins apart, so their four
                     // taps lie in THREE consecutive bins starting at the smaller left index: 3 loads
@@ -354,11 +396,11 @@ bp_tile_kernel(const BqParams P)
                     if (cs.x >= 0.0f) {
 #pragma unroll
                         for (int m = 0; m + 1 < PPT; m += 2)
-                            bq_pair<V, SB>(acc[m], acc[m + 1], fmaf(kyf[m], cs.x, vb), fmaf(kyf[m + 1], cs.x, vb), seg);
+                            bq_pair<V, SB, MT>(acc[m], acc[m + 1], fmaf(kyf[m], cs.x, vb), fmaf(kyf[m + 1], cs.x, vb), seg, k);
                     } else {
 #pragma unroll
                         for (int m = 0; m + 1 < PPT; m += 2)
-                            bq_pair<V, SB>(acc[m + 1], acc[m], fmaf(kyf[m + 1], cs.x, vb), fmaf(kyf[m], cs.x, vb), seg);
+                            bq_pair<V, SB, MT>(acc[m + 1], acc[m], fmaf(kyf[m + 1], cs.x, vb), fmaf(kyf[m], cs.x, vb), seg, k);
                     }
                     continue;
                 }
@@ -378,7 +420,11 @@ bp_tile_kernel(const BqParams P)
                     tr[m] = LD::template ld<SB * 4>(ad[m]);
                 }
 #pragma unroll
-                for (int m = 0; m < PPT; ++m) bq_tap(acc[m], tl[m], tr[m], 1.0f - w[m], w[m]);
+                for (int m = 0; m < PPT; ++m) {
+                    float wl, wr;
+                    bq_w2<MT>(k, w[m], wl, wr);
+                    bq_tap(acc[m], tl[m], tr[m], wl, wr);
+                }
             }
             __syncwarp();
             if (lane == 0) bq_mbar_arrive(&empty[bi]);
@@ -593,14 +639,22 @@ size_t scd_sino_il_bytes(const scd_geom *g, int batch)
     return need + 256;
 }
 
-template <int V, int LPR, int PPT, bool IL>
-static int bq_launch_t(const BqParams &P, const BqConfig &c, cudaStream_t st, int device)
+template <int V, int LPR, int PPT, bool IL, bool MT>
+static int bq_launch_mt(const BqParams &P, const BqConfig &c, cudaStream_t st, int device)
 {
     static ScdSmemAttr attr = {};        // per instantiation
-    SCD_CUDA(scd_ensure_smem(bp_tile_kernel<V, LPR, PPT, IL>, attr, device, c.smem));
-    SCD_CUDA(scd_launch_kernel(bp_tile_kernel<V, LPR, PPT, IL>, c.grid, dim3(BQ_THREADS), c.smem, st, 0, P));
+    SCD_CUDA(scd_ensure_smem(bp_tile_kernel<V, LPR, PPT, IL, MT>, attr, device, c.smem));
+    SCD_CUDA(scd_launch_kernel(bp_tile_kernel<V, LPR, PPT, IL, MT>, c.grid, dim3(BQ_THREADS), c.smem, st, 0, P));
     SCD_LAUNCH_CHECK("bp_tile_kernel");
     return 0;
+}
+
+// the pixel-driven or the matched march, by the geometry
+template <int V, int LPR, int PPT, bool IL>
+static int bq_launch_t(const BqParams &P, const BqConfig &c, cudaStream_t st, const scd_geom *g)
+{
+    return g->matched ? bq_launch_mt<V, LPR, PPT, IL, true>(P, c, st, g->device)
+                      : bq_launch_mt<V, LPR, PPT, IL, false>(P, c, st, g->device);
 }
 
 // banded output: every tile lies inside one band and every band has somewhere to go
@@ -647,13 +701,13 @@ int scd_launch_bp_il(const scd_geom *g, const float *sino_il, float *out, int ba
     if (ep.il) {
         if (c.V == 2 || ep.n_bands) { scd_set_error("scd_bp: interleaved images need groups of 1 or >= 4 samples and no bands"); return SCD_E_INVALID; }
         if (ep.mode == 1 && (!ep.add1 || !ep.out2 || (ep.beta && !ep.add2))) { scd_set_error("scd_bp: direction step needs r, p"); return SCD_E_INVALID; }
-#define BQ_CASE_IL(LL, PP) if (c.V == 4 && c.LPR == LL && c.PPT == PP) return bq_launch_t<4, LL, PP, true>(P, c, st, g->device);
+#define BQ_CASE_IL(LL, PP) if (c.V == 4 && c.LPR == LL && c.PPT == PP) return bq_launch_t<4, LL, PP, true>(P, c, st, g);
         BQ_CASE_IL(1, 1) BQ_CASE_IL(1, 2) BQ_CASE_IL(2, 1) BQ_CASE_IL(2, 2) BQ_CASE_IL(2, 4) BQ_CASE_IL(4, 2) BQ_CASE_IL(4, 4)
 #undef BQ_CASE_IL
-        if (c.V == 1 && c.PPT == 1) return bq_launch_t<1, 1, 1, true>(P, c, st, g->device);      // one sample per group
-        if (c.V == 1 && c.PPT == 2) return bq_launch_t<1, 1, 2, true>(P, c, st, g->device);
+        if (c.V == 1 && c.PPT == 1) return bq_launch_t<1, 1, 1, true>(P, c, st, g);      // one sample per group
+        if (c.V == 1 && c.PPT == 2) return bq_launch_t<1, 1, 2, true>(P, c, st, g);
     }
-#define BQ_CASE(VV, LL, PP) if (c.V == VV && c.LPR == LL && c.PPT == PP) return bq_launch_t<VV, LL, PP, false>(P, c, st, g->device);
+#define BQ_CASE(VV, LL, PP) if (c.V == VV && c.LPR == LL && c.PPT == PP) return bq_launch_t<VV, LL, PP, false>(P, c, st, g);
     BQ_CASE(1, 1, 1) BQ_CASE(1, 1, 2) BQ_CASE(2, 1, 1) BQ_CASE(2, 1, 2) BQ_CASE(4, 1, 1) BQ_CASE(4, 1, 2)
     BQ_CASE(4, 2, 1) BQ_CASE(4, 2, 2) BQ_CASE(4, 2, 4) BQ_CASE(4, 4, 2) BQ_CASE(4, 4, 4)
 #undef BQ_CASE

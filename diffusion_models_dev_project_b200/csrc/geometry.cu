@@ -61,8 +61,23 @@ extern "C" int scd_geom_create(const scd_geom_desc *d, scd_geom_t **out)
 
 extern "C" int scd_geom_create_weighted(const scd_geom_desc *d, const double *wts, scd_geom_t **out)
 {
+    return scd_geom_create_ex(d, wts, 0, out);
+}
+
+extern "C" int scd_geom_create_ex(const scd_geom_desc *d, const double *wts, uint32_t flags, scd_geom_t **out)
+{
     if (!d || !out) { scd_set_error("scd_geom_create: null argument"); return SCD_E_INVALID; }
     *out = nullptr;
+    if (flags & ~(uint32_t)SCD_GEOM_MATCHED_ADJOINT) {
+        scd_set_error("scd_geom_create_ex: unknown flag bits 0x%x", (unsigned)(flags & ~(uint32_t)SCD_GEOM_MATCHED_ADJOINT));
+        return SCD_E_INVALID;
+    }
+    // the matched backprojector's hat has half-width max(|cos|, |sin|) * dx/ds bins; its three taps around round(v)
+    // cover it only while that stays below 1.5
+    if ((flags & SCD_GEOM_MATCHED_ADJOINT) && d->dx > 0 && d->ds > 0 && !(d->dx / d->ds < 1.5)) {
+        scd_set_error("scd_geom_create_ex: the matched adjoint needs dx/ds < 1.5 (got dx=%g ds=%g)", d->dx, d->ds);
+        return SCD_E_INVALID;
+    }
     if (wts && d->n_angles >= 1) {
         bool all_one = true;
         for (int i = 0; i < d->n_angles; ++i) {
@@ -106,6 +121,7 @@ extern "C" int scd_geom_create_weighted(const scd_geom_desc *d, const double *wt
     g->x_min = d->x_min; g->y_min = d->y_min; g->dx = d->dx;
     g->s_min = d->s_min; g->ds = d->ds; g->adj_scale = d->adj_scale;
     g->device = dev;
+    g->matched = (flags & SCD_GEOM_MATCHED_ADJOINT) ? 1 : 0;
     { const char *e = getenv("SCD_FP_SOURCE"); if (e && !strcmp(e, "packed")) g->tune_fp_source = 1; }   // A/B runs
     { static std::atomic<unsigned long long> next_id{1}; g->id = next_id.fetch_add(1); }
     g->sm_count = prop.multiProcessorCount;

@@ -144,6 +144,8 @@ struct scd_geom {
     int tune_fp_source;   // 1: force the packed-copy path of the projector (A/B runs, tests)
     // sample-interleaved sinogram rows (bp_tile.cu): il_padl zero bins, n_det bins, zero bins up to il_nb
     int il_padl, il_nb;
+    // SCD_GEOM_MATCHED_ADJOINT: every backprojection runs the matched march of bp_tile (exact transpose of A)
+    int matched;
 };
 
 // ------------------------------------------------------------ launchers ----

@@ -30,7 +30,7 @@ def _stream_ptr(device):
 class _GeomHandle:
     """Owns one ``scd_geom_t*`` (device tables) for one CUDA device."""
 
-    def __init__(self, geom: ParallelBeamGeometry2D, adj_scale: float, device: torch.device):
+    def __init__(self, geom: ParallelBeamGeometry2D, adj_scale: float, device: torch.device, matched: bool = False):
         lib = _lib.load()
         ang = np.ascontiguousarray(geom.angles, dtype=np.float64)
         desc = _lib.GeomDesc(
@@ -38,15 +38,20 @@ class _GeomHandle:
             n_angles=geom.n_angles, angles=ang.ctypes.data_as(C.POINTER(C.c_double)),
             n_det=geom.n_det, s_min=geom.s_min, ds=geom.ds, adj_scale=adj_scale)
         h = C.c_void_p()
+        w = None
+        if geom.angle_weights is not None:
+            w = np.ascontiguousarray(geom.angle_weights, dtype=np.float64)
+            if w.shape != (geom.n_angles,):
+                raise ValueError('angle_weights: expected shape (%d,), got %r' % (geom.n_angles, w.shape))
+        wp = w.ctypes.data_as(C.POINTER(C.c_double)) if w is not None else None
         with torch.cuda.device(device):
-            if geom.angle_weights is None:
+            if matched:
+                _lib.check(lib.scd_geom_create_ex(C.byref(desc), wp, _lib.SCD_GEOM_MATCHED_ADJOINT, C.byref(h)),
+                           'scd_geom_create_ex')
+            elif w is None:
                 _lib.check(lib.scd_geom_create(C.byref(desc), C.byref(h)), 'scd_geom_create')
             else:
-                w = np.ascontiguousarray(geom.angle_weights, dtype=np.float64)
-                if w.shape != (geom.n_angles,):
-                    raise ValueError('angle_weights: expected shape (%d,), got %r' % (geom.n_angles, w.shape))
-                _lib.check(lib.scd_geom_create_weighted(C.byref(desc), w.ctypes.data_as(C.POINTER(C.c_double)),
-                                                        C.byref(h)), 'scd_geom_create_weighted')
+                _lib.check(lib.scd_geom_create_weighted(C.byref(desc), wp, C.byref(h)), 'scd_geom_create_weighted')
         self.ptr = h
         self.device = device
         self._lib = lib
@@ -63,7 +68,9 @@ class _GeomHandle:
 class _TrafoFn(torch.autograd.Function):
     """y = A x.  Backward: the unweighted transpose A^T g = A*(g)/c_w (ODL
     ``OperatorFunction`` convention, SURVEY.md §8b).  With view weights w_i, A* carries them and the
-    transpose is A*(g / w)/c_w (c_w: the mean cell)."""
+    transpose is A*(g / w)/c_w (c_w: the mean cell).  With the pixel-driven A* this pairing is off by the
+    matched/unmatched gap; with ``adjoint='matched'`` (and ``adjoint_scaling='dphi'``) it is the exact
+    transpose J^T g of the Joseph matrix."""
 
     @staticmethod
     def forward(ctx, x, rt):
@@ -128,6 +135,16 @@ class B200RayTrafo(BaseRayTrafo):
         continuous weighted adjoint (kappa = 1 of SURVEY.md §8c), ``'dphi/ds'``
         the alternative kappa = 1/ds convention.  ``dphi`` is the mean angle cell and
         ``w_i`` the view weights of the geometry (1 for a uniform partition).
+    adjoint : {'pixel', 'matched'}
+        ``'pixel'`` (default): A* is the pixel-driven linear-interpolation backprojector (ODL / ASTRA's
+        unmatched adjoint, the reference's ``SimpleTrafo``).  ``'matched'``: A* is the exact transpose of the
+        Joseph projector, ``A* = (adj_scale/dphi) c_w J^T diag(w)`` with ``c_w = dphi*ds/dx^2`` (the reference's
+        ``MatmulRayTrafo``), evaluated by the same kernel with a normalised hat of half-width
+        ``dx max(|cos|,|sin|)/ds`` bins (``scd_geom_create_ex`` with ``SCD_GEOM_MATCHED_ADJOINT``).  Every
+        backprojection of the operator uses it -- ``trafo_adjoint``, ``normal_apply``, ``cg_solve``, ``dds_step``,
+        the fused adaptation objective, ``fbp`` -- so ``(I + gamma A*A)`` is symmetric positive definite and the
+        gradient autograd returns through ``trafo`` is the exact transpose ``J^T g``.  ``A`` is the same either
+        way.  Needs ``dx/ds < 1.5`` (every geometry ``SimpleTrafo`` derives has ``dx/ds`` just above 1).
     geometry : ParallelBeamGeometry2D, optional
         An explicit geometry (angle list and view weights, detector partition, pixel size,
         domain offset) instead of the one ``SimpleTrafo`` derives from ``(im_shape, num_angles)``;
@@ -137,9 +154,13 @@ class B200RayTrafo(BaseRayTrafo):
         limited-angle (missing wedge) geometry of ``ParallelBeamGeometry2D.from_angle_range``.
     """
 
-    def __init__(self, im_shape, num_angles, impl='b200', adjoint_scaling='dphi', geometry=None, angle_range=None):
+    def __init__(self, im_shape, num_angles, impl='b200', adjoint_scaling='dphi', geometry=None, angle_range=None,
+                 adjoint='pixel'):
         if impl not in ('b200', 'odl', 'iradon'):
             raise NotImplementedError(impl)
+        if adjoint not in ('pixel', 'matched'):
+            raise ValueError("adjoint must be 'pixel' or 'matched' (got %r)" % (adjoint,))
+        self.adjoint = adjoint
         if geometry is not None and angle_range is not None:
             raise ValueError('pass either geometry or angle_range')
         if geometry is not None:
@@ -179,7 +200,8 @@ class B200RayTrafo(BaseRayTrafo):
             with self._hlock:
                 h = self._handles.get(idx)
                 if h is None:
-                    h = _GeomHandle(self.geometry, self.adj_scale, torch.device('cuda', idx))
+                    h = _GeomHandle(self.geometry, self.adj_scale, torch.device('cuda', idx),
+                                    matched=self.adjoint == 'matched')
                     self._handles[idx] = h
         return h
 
@@ -555,5 +577,10 @@ class B200RayTrafo(BaseRayTrafo):
         On a weighted geometry the backprojector sums view ``i`` with ``dphi * w_i``, its angular cell: the
         FBP quadrature of a non-uniform view set.  On a wedge the result is the truncated FBP -- the inverse
         Radon formula restricted to the measured angles -- not a limited-angle reconstruction: the missing
-        wedge stays missing (streaks and lost edges along it)."""
+        wedge stays missing (streaks and lost edges along it).
+
+        On a matched operator (``adjoint='matched'``) the filtered rows are backprojected with the normalised
+        hat of the matched A*, i.e. by ``c_w J^T``: the result is ``(dphi/dx^2) J^T diag(w) (ds * ramp_filter(y))``,
+        which on the uniform partition of [0, pi) is ``J^T filter_sinogram(y) / dx^2`` with the reference's
+        ``filter_sinogram``."""
         return self._bp(self.ramp_filter(observation), self.geometry.dphi)

@@ -77,6 +77,8 @@ class AngleShardedRayTrafo:
     ``normal_op(gamma)`` -> callable for :func:`..utils.cg.cg` (tensor-op recurrences on replicated vectors).
 
     Inference-only: the sharded operators do not record autograd graphs and raise if an input requires grad.
+    Every backprojection runs on ``base``: a base built with ``adjoint='matched'`` makes the sharded A* the
+    exact transpose as well (``adjoint`` reports the base's setting).
     """
 
     def __init__(self, base, group=None, chunk: int = 256, reduce: str = 'nccl', multicast=None, balance: str = 'cost'):
@@ -104,6 +106,10 @@ class AngleShardedRayTrafo:
     @property
     def angles(self):
         return self.base.angles
+
+    @property
+    def adjoint(self):
+        return getattr(self.base, 'adjoint', 'pixel')
 
     # ---------------------------------------------------------------- A ----
     def trafo(self, x: Tensor) -> Tensor:

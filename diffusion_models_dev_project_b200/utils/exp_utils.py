@@ -4,7 +4,7 @@
 ``trafo_name='simple_trafo'`` whatever ``forward_op.impl`` says (there is one
 implementation); the optional keys ``forward_op.angle_range`` (a limited-angle wedge)
 and ``forward_op.angles`` (an explicit, possibly non-uniform view set) select other
-angle sets.  ``get_standard_sampler`` keeps the reference's signature but
+angle sets, and ``forward_op.adjoint`` (``'pixel'`` or ``'matched'``) the backprojector.  ``get_standard_sampler`` keeps the reference's signature but
 builds the DDPM/'dds' sampler correctly: the reference passes an
 ``init_chain_fn`` keyword ``BaseSampler`` does not accept and therefore raises
 (exp_utils.py:214-221, see SURVEY.md §3.1); only the branch the hot path needs
@@ -46,11 +46,15 @@ def _optional(ns, key):
 def get_standard_ray_trafo(config):
     """``forward_op.angle_range = (min, max)`` (radians): ``num_angles`` cell-centred views on ``[min, max)``.
     ``forward_op.angles`` (radians): exactly these views, weighted by their angular cells (``num_angles`` may be
-    omitted; if given it must equal their count).  Without either key: ``num_angles`` views on ``[0, pi)``."""
+    omitted; if given it must equal their count).  Without either key: ``num_angles`` views on ``[0, pi)``.
+    ``forward_op.adjoint``: ``'pixel'`` (default, the pixel-driven A* of ``SimpleTrafo``) or ``'matched'`` (the exact
+    transpose of the projector, as the reference's ``MatmulRayTrafo``); see :class:`B200RayTrafo`."""
     fo = config.forward_op
     if fo.trafo_name.lower() != 'simple_trafo':
         raise NotImplementedError(fo.trafo_name)
     im_shape = (config.data.im_size, config.data.im_size)
+    adjoint = _optional(fo, 'adjoint')
+    adjoint = 'pixel' if adjoint is None else adjoint
     angle_range = _optional(fo, 'angle_range')
     angles = _optional(fo, 'angles')
     if angle_range is not None and angles is not None:
@@ -60,11 +64,11 @@ def get_standard_ray_trafo(config):
         num_angles = _optional(fo, 'num_angles')
         if num_angles is not None and int(num_angles) != geom.n_angles:
             raise ValueError('forward_op.num_angles = %d but %d angles are given' % (int(num_angles), geom.n_angles))
-        return B200RayTrafo(im_shape=im_shape, num_angles=geom.n_angles, impl=fo.impl, geometry=geom)
+        return B200RayTrafo(im_shape=im_shape, num_angles=geom.n_angles, impl=fo.impl, geometry=geom, adjoint=adjoint)
     if angle_range is not None:
         return B200RayTrafo(im_shape=im_shape, num_angles=fo.num_angles, impl=fo.impl,
-                            angle_range=tuple(float(a) for a in angle_range))
-    return B200RayTrafo(im_shape=im_shape, num_angles=fo.num_angles, impl=fo.impl)
+                            angle_range=tuple(float(a) for a in angle_range), adjoint=adjoint)
+    return B200RayTrafo(im_shape=im_shape, num_angles=fo.num_angles, impl=fo.impl, adjoint=adjoint)
 
 
 def get_data_from_ground_truth(ground_truth, ray_trafo, white_noise_rel_stddev):

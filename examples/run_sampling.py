@@ -11,6 +11,7 @@ data-consistency path, not a trained prior), a small LoRA injector instead of th
     python examples/run_sampling.py --mode adapted --num_steps 10 --num_optim_step 2 --add_cg
     python examples/run_sampling.py --num_steps 20 --angle_range 0 90        # limited angle: a 90 degree wedge
     python examples/run_sampling.py --num_steps 20 --angles_file views.txt   # sparse / non-uniform views
+    python examples/run_sampling.py --num_steps 20 --adjoint matched         # A* = exact transpose of A
 """
 import argparse
 import os
@@ -61,6 +62,9 @@ def parse():
     p.add_argument('--angles_file', default=None,
                    help='text file of view angles in degrees (whitespace or newline separated), weighted by their '
                         'angular cells; replaces --num_angles')
+    p.add_argument('--adjoint', default='pixel', choices=['pixel', 'matched'],
+                   help="backprojector: 'pixel' (pixel-driven, SimpleTrafo's) or 'matched' (exact transpose of the "
+                        "Joseph projector, MatmulRayTrafo's)")
     p.add_argument('--batch_size', type=int, default=1)
     p.add_argument('--num_images', type=int, default=1)
     p.add_argument('--unet', default='small', choices=['small', 'aapm', 'blur'],
@@ -73,7 +77,7 @@ def parse():
 def main():
     args = parse()
     device = torch.device('cuda')
-    forward_op = NS(trafo_name='simple_trafo', num_angles=args.num_angles, impl='b200')
+    forward_op = NS(trafo_name='simple_trafo', num_angles=args.num_angles, impl='b200', adjoint=args.adjoint)
     if args.angle_range is not None and args.angles_file is not None:
         raise SystemExit('give --angle_range or --angles_file, not both')
     if args.angle_range is not None:

@@ -5,7 +5,8 @@
  * SCD / DDS reverse sampler of educating-dip/diffusion_models_dev_project:
  *
  *   A   parallel-beam ray transform, ray-driven Joseph projector
- *   A*  pixel-driven linear-interpolation backprojector (weighted adjoint)
+ *   A*  pixel-driven linear-interpolation backprojector (weighted adjoint), or
+ *       the exact transpose of A (scd_geom_create_ex, SCD_GEOM_MATCHED_ADJOINT)
  *   CG  batched conjugate gradient on (I + gamma A*A) x = rhs
  *   Tweedie + rhs, DDIM update (DDPM schedule)
  *
@@ -75,6 +76,21 @@ int scd_geom_create(const scd_geom_desc *desc, scd_geom_t **out);
  * scd_adapt_bwd stays unweighted: it is the transpose of A.
  * angle_weights == NULL, or every entry exactly 1.0: identical to scd_geom_create.                      */
 int scd_geom_create_weighted(const scd_geom_desc *desc, const double *angle_weights, scd_geom_t **out);
+
+/* Geometry with options.  scd_geom_create_weighted(desc, w, out) is scd_geom_create_ex(desc, w, 0, out); flag
+ * bits other than the ones below are rejected (SCD_E_INVALID, *out = NULL, nothing allocated).
+ *   SCD_GEOM_MATCHED_ADJOINT  A* is the exact transpose of the Joseph projector A instead of the pixel-driven
+ *       linear-interpolation backprojector: with c_w = dphi*ds/dx^2 and J the matrix of scd_fp,
+ *           A* y = (adj_scale/dphi) * c_w * J^T diag(w) y
+ *                = adj_scale * sum_i w_i sum_j k_i max(0, 1 - k_i |j - v_i(x)|) y_ij,   k_i = ds / (dx max(|cos|,|sin|))
+ *       (the pixel-driven sum with the unit hat replaced by one of unit area and half-width 1/k_i; the reference's
+ *       MatmulRayTrafo).  Every backprojection of the geometry uses it: scd_bp, scd_bp_il, scd_bp_ilimg,
+ *       scd_bp_host, scd_bp_banded, scd_bp_il_banded, and those inside scd_cg, scd_dds_step, scd_adapt_fwd/bwd.
+ *       (I + gamma A*A) is then symmetric positive definite, and the gradient backprojection of scd_adapt_bwd
+ *       with trafo_grad_scale = adj_scale/c_w is the exact gradient.  scd_fp is unchanged.  Needs dx/ds < 1.5
+ *       (the hat then spans at most three detector bins); larger ratios are rejected.                      */
+#define SCD_GEOM_MATCHED_ADJOINT 0x1u
+int scd_geom_create_ex(const scd_geom_desc *desc, const double *angle_weights, uint32_t flags, scd_geom_t **out);
 int scd_geom_destroy(scd_geom_t *g);
 
 /* A: forward projection of angles [angle_lo, angle_hi) (rows outside that
