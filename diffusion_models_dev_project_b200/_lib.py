@@ -49,14 +49,21 @@ SIGNATURES = {
     "scd_img_il_unpack": (C.c_int, [C.c_void_p, _F, _F, C.c_int, C.c_void_p]),
     "scd_fp_ilimg": (C.c_int, [C.c_void_p, _F, _F, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "scd_bp_ilimg": (C.c_int, [C.c_void_p, _F, _F, C.c_int, C.c_int, C.c_int, C.c_float, _F, C.c_float, C.c_void_p]),
+    "scd_sino_weights_pack": (C.c_int, [C.c_void_p, _F, _F, C.c_int, C.c_void_p]),
+    "scd_fp_il_w": (C.c_int, [C.c_void_p, _F, _F, _F, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "scd_fp_ilimg_w": (C.c_int, [C.c_void_p, _F, _F, _F, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "scd_cg_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
     "scd_cg": (C.c_int, [C.c_void_p, _F, _F, C.c_double, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "scd_cg_w": (C.c_int, [C.c_void_p, _F, _F, _F, C.c_double, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "scd_tweedie_rhs": (C.c_int, [_F, _F, _F, _F, _F, C.c_int, C.c_double, _F, _F, C.c_int, C.c_int64, C.c_void_p]),
     "scd_ddim": (C.c_int, [_F, _F, _F, _F, _F, _F, C.c_int, C.c_double, _F, C.c_int, C.c_int64, C.c_void_p]),
     "scd_dds_step": (C.c_int, [C.c_void_p, _F, _F, _F, _F, _F, _F, _F, C.c_int, C.c_double, C.c_double,
                                C.c_int, _F, _F, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "scd_dds_step_w": (C.c_int, [C.c_void_p, _F, _F, _F, _F, _F, _F, _F, _F, C.c_int, C.c_double, C.c_double,
+                                 C.c_int, _F, _F, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "scd_residual_sq_blocks": (C.c_int, [C.c_int64]),
     "scd_residual_sq": (C.c_int, [_F, _F, _F, _F, C.c_int64, C.c_void_p]),
+    "scd_residual_sq_w": (C.c_int, [_F, _F, _F, _F, _F, C.c_int64, C.c_void_p]),
     "scd_tv_blocks": (C.c_int, [C.c_int, C.c_int]),
     "scd_tv_loss": (C.c_int, [_F, _F, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "scd_tv_grad": (C.c_int, [_F, _F, C.c_int, C.c_int, C.c_int, C.c_void_p]),
@@ -65,6 +72,10 @@ SIGNATURES = {
                                 _F, _F, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "scd_adapt_bwd": (C.c_int, [C.c_void_p, _F, _F, _F, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double, C.c_double,
                                 _F, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "scd_adapt_fwd_w": (C.c_int, [C.c_void_p, _F, _F, _F, _F, _F, _F, _F, _F, C.c_int, C.c_double, C.c_int, C.c_int,
+                                  C.c_double, _F, _F, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "scd_adapt_bwd_w": (C.c_int, [C.c_void_p, _F, _F, _F, _F, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double,
+                                  C.c_double, _F, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "scd_ramp_filter": (C.c_int, [C.c_void_p, _F, _F, C.c_int, C.c_void_p]),
     "scd_bp_banded": (C.c_int, [C.c_void_p, _F, C.c_int, C.c_int, C.c_int, C.c_float, C.POINTER(C.c_void_p), C.c_int, C.c_int,
                                 C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -21,6 +21,10 @@
 //   finally  gr <- gr + gp + 2 grho r_0;   d loss/d xhat0 = gx - gamma A*(A gr)   (start value + right-hand side)
 //            d loss/d s = -(std_t/mean_t) * d loss/d xhat0
 //
+// Measurement weights (scd_adapt_fwd_w / _bwd_w): every op application projects with W (w_il, packed), and the
+// loss is mean(W (A xhat - y)^2) + lambda tv: the residual kept for the sweep is r_w = W (A xhat - y), whose plain
+// transpose backprojection is the gradient of the weighted data term, so the sweep itself is unchanged.
+//
 // All buffers live in one caller-provided workspace (scd_adapt_workspace_bytes), which carries the saved vectors
 // from scd_adapt_fwd to scd_adapt_bwd.  No allocation, no synchronisation, no host read-back: both calls are
 // CUDA-graph capturable.
@@ -310,6 +314,7 @@ extern "C" size_t scd_adapt_workspace_bytes(const scd_geom_t *g, int batch, int 
 namespace {
 struct AdCtx {
     const scd_geom *g; AdLayout L; char *w; int batch; cudaStream_t st; float gs; int64_t numel; dim3 grid;
+    const float *w_il;     // packed measurement weights of op or NULL
     float *img(size_t off, size_t k = 0) const { return (float *)(w + off + k * L.img); }
     float *part(int k) const { return (float *)(w + L.off_part) + (size_t)k * L.stride * batch; }
     float *scal(int which, size_t k) const { return (float *)(w + L.off_scal) + ((size_t)which * std::max<size_t>(L.K, 1) + k) * batch; }
@@ -319,7 +324,8 @@ struct AdCtx {
            float *out2, float *dot_part, int dot_with_add1) const
     {
         float *q = (float *)(w + L.off_q);
-        int rc = scd_launch_fp(g, v, nullptr, q, batch, 0, g->n_angles, w + L.off_pack, scd_fp_scratch_need(g, batch), st, nullptr);
+        int rc = scd_launch_fp(g, v, nullptr, q, batch, 0, g->n_angles, w + L.off_pack, scd_fp_scratch_need(g, batch), st, nullptr,
+                               w_il);
         if (rc) return rc;
         BpEpilogue e;
         e.c_acc = c_acc; e.add1 = add1; e.c1 = c1; e.add2 = add2; e.c2 = c2; e.out2 = out2;
@@ -329,9 +335,11 @@ struct AdCtx {
 };
 
 int ad_setup(AdCtx &c, const scd_geom_t *g, int batch, int n_iter, int dc_type, void *work, size_t work_bytes, double gamma,
-             void *stream, const char *who)
+             void *stream, const char *who, const float *w_il)
 {
     if (n_iter < 0 || dc_type < 0 || dc_type > 2) { scd_set_error("%s: bad n_iter / dc_type", who); return SCD_E_INVALID; }
+    if (((uintptr_t)w_il & 127) != 0) { scd_set_error("%s: w_il must be 128-byte aligned", who); return SCD_E_INVALID; }
+    c.w_il = w_il;
     if (((uintptr_t)work & 255) != 0) { scd_set_error("%s: workspace must be 256-byte aligned", who); return SCD_E_INVALID; }
     c.g = g; c.L = ad_layout(g, batch, dc_type == 0 ? n_iter : 0); c.w = (char *)work; c.batch = batch; c.st = (cudaStream_t)stream;
     if (work_bytes < c.L.total) {
@@ -358,12 +366,22 @@ extern "C" int scd_adapt_fwd(const scd_geom_t *g, const float *x, const float *s
                              double tv_lambda, float *loss, float *xhat_out, int batch, void *work, size_t work_bytes,
                              void *stream)
 {
+    return scd_adapt_fwd_w(g, x, s, atb, y, nullptr, nullptr, t, abar, n_table, gamma, n_iter, dc_type, tv_lambda, loss,
+                           xhat_out, batch, work, work_bytes, stream);
+}
+
+extern "C" int scd_adapt_fwd_w(const scd_geom_t *g, const float *x, const float *s, const float *atb, const float *y,
+                               const float *w, const float *w_il, const float *t, const float *abar, int n_table,
+                               double gamma, int n_iter, int dc_type, double tv_lambda, float *loss, float *xhat_out,
+                               int batch, void *work, size_t work_bytes, void *stream)
+{
+    if (!w != !w_il) { scd_set_error("scd_adapt_fwd_w: give both w and w_il, or neither"); return SCD_E_INVALID; }
     if (!g || !x || !s || !y || !t || !abar || !loss || !work || (dc_type != 2 && !atb)) {
         scd_set_error("scd_adapt_fwd: null argument"); return SCD_E_INVALID;
     }
     if (batch <= 0) { scd_set_error("scd_adapt_fwd: empty batch"); return SCD_E_INVALID; }
     AdCtx c;
-    int rc = ad_setup(c, g, batch, n_iter, dc_type, work, work_bytes, gamma, stream, "scd_adapt_fwd");
+    int rc = ad_setup(c, g, batch, n_iter, dc_type, work, work_bytes, gamma, stream, "scd_adapt_fwd", w_il);
     if (rc) return rc;
     const AdLayout &L = c.L;
     const int K = (int)L.K, ps = (int)L.stride;
@@ -405,7 +423,7 @@ extern "C" int scd_adapt_fwd(const scd_geom_t *g, const float *x, const float *s
     float *respart = (float *)(c.w + L.off_respart), *tvpart = (float *)(c.w + L.off_tvpart);
     if ((rc = scd_launch_fp(g, xk, ax, nullptr, batch, 0, g->n_angles, c.w + L.off_pack, scd_fp_scratch_need(g, batch), c.st, nullptr))) return rc;
     const int64_t n_res = (int64_t)g->n_angles * g->n_det * batch;
-    if ((rc = scd_residual_sq(ax, y, res, respart, n_res, stream))) return rc;
+    if ((rc = scd_launch_residual_sq(ax, y, w, res, respart, n_res, c.st))) return rc;
     if ((rc = scd_tv_loss(xk, tvpart, batch, g->n0, g->n1, stream))) return rc;
     SCD_CUDA(scd_launch_kernel(adapt_loss_kernel, dim3(1), dim3(AD_THREADS), 0, c.st, 0, (const float *)respart, L.res_blocks,
                                (const float *)tvpart, L.tv_blocks * batch, 1.0f / (float)n_res, (float)tv_lambda, loss));
@@ -417,16 +435,26 @@ extern "C" int scd_adapt_bwd(const scd_geom_t *g, const float *grad_loss, const 
                              double gamma, int n_iter, int dc_type, double tv_lambda, double trafo_grad_scale,
                              float *grad_s, int batch, void *work, size_t work_bytes, void *stream)
 {
+    return scd_adapt_bwd_w(g, grad_loss, nullptr, t, abar, n_table, gamma, n_iter, dc_type, tv_lambda, trafo_grad_scale,
+                           grad_s, batch, work, work_bytes, stream);
+}
+
+extern "C" int scd_adapt_bwd_w(const scd_geom_t *g, const float *grad_loss, const float *w_il, const float *t,
+                               const float *abar, int n_table, double gamma, int n_iter, int dc_type, double tv_lambda,
+                               double trafo_grad_scale, float *grad_s, int batch, void *work, size_t work_bytes,
+                               void *stream)
+{
     if (!g || !t || !abar || !grad_s || !work) { scd_set_error("scd_adapt_bwd: null argument"); return SCD_E_INVALID; }
     if (batch <= 0) { scd_set_error("scd_adapt_bwd: empty batch"); return SCD_E_INVALID; }
     AdCtx c;
-    int rc = ad_setup(c, g, batch, n_iter, dc_type, work, work_bytes, gamma, stream, "scd_adapt_bwd");
+    int rc = ad_setup(c, g, batch, n_iter, dc_type, work, work_bytes, gamma, stream, "scd_adapt_bwd", w_il);
     if (rc) return rc;
     const AdLayout &L = c.L;
     const int K = (int)L.K, ps = (int)L.stride;
     float *xk = c.img(L.off_x), *gx = c.img(L.off_gx), *val = c.img(L.off_val);
     float *res = (float *)(c.w + L.off_res);
-    // gx = d loss / d xhat = (2/N) A*(res)/c_w + lambda d tv/d xhat     (gradient of A under ODL's pairing)
+    // gx = d loss / d xhat = (2/N) A*(res)/c_w + lambda d tv/d xhat     (gradient of A under ODL's pairing; res is
+    // W (A xhat - y) when the forward call was weighted)
     float *tvg = c.img(L.off_gd);                                        // free until the sweep needs gd
     if ((rc = scd_tv_grad(xk, tvg, batch, g->n0, g->n1, stream))) return rc;
     const double n_res = (double)g->n_angles * g->n_det * batch;

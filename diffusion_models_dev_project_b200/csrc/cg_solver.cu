@@ -16,6 +16,9 @@
 //   cg_update_xr_il   alpha = rr/<p,d>;  x += alpha p;  r -= alpha d;  partial ||r||^2
 // Batches of 2 samples (and batch 1 when n1 is not a multiple of 4) keep the packed-copy sequence:
 // fp_packq (p-update fused), fp_march, bp_tile(+axpy,+<p,d>), cg_update_xr (the last p-update is skipped).
+// Measurement weights (the _w entry points): op(v) = v + gamma*A*(W A v).  W, packed once into the layout of q
+// (scd_sino_weights_pack), multiplies the projector's interleaved output before the recurrence q = A r + beta q;
+// both are linear, so the recurrence stays exact.  No other launch changes.
 #include "scd_internal.cuh"
 #include <algorithm>
 #include <cstring>
@@ -73,7 +76,7 @@ extern "C" size_t scd_cg_workspace_bytes(const scd_geom_t *g, int batch)
 
 int scd_cg_run(const scd_geom *g, const float *x_in, float *x, const float *rhs, float gamma,
                int n_iter, int batch, void *work, size_t work_bytes, cudaStream_t st,
-               const FpPrologue *first)
+               const FpPrologue *first, const float *w_il)
 {
     if (!g || !x || !x_in || !rhs || !work) { scd_set_error("scd_cg: null argument"); return SCD_E_INVALID; }
     if (batch <= 0) return 0;
@@ -106,7 +109,7 @@ int scd_cg_run(const scd_geom *g, const float *x_in, float *x, const float *rhs,
 
     // r = rhs - x - gamma A*(A x);  p = r;  rr = ||r||^2
     // (the Tweedie step that produces x_in and rhs may be fused into this projection's pack pass)
-    if ((rc = scd_launch_fp(g, x_in, q_user, q_il, batch, 0, g->n_angles, pack, L.pack_bytes, st, first))) return rc;
+    if ((rc = scd_launch_fp(g, x_in, q_user, q_il, batch, 0, g->n_angles, pack, L.pack_bytes, st, first, w_il))) return rc;
     BpEpilogue e0;
     e0.c_acc = -gs; e0.add1 = x_in; e0.c1 = -1.f; e0.add2 = rhs; e0.c2 = 1.f;
     e0.out2 = p; e0.dot_part = rr_a; e0.dot_stride = ps; e0.dot_with_add1 = 0;
@@ -124,7 +127,8 @@ int scd_cg_run(const scd_geom *g, const float *x_in, float *x, const float *rhs,
             up.rr_old_part = rr_new; up.rr_old_n = rr_prev_n;       // and the one before it
             up.part_stride = ps;
         }
-        if ((rc = scd_launch_fp(g, p, q_user, q_il, batch, 0, g->n_angles, pack, L.pack_bytes, st, it > 0 ? &up : nullptr))) return rc;
+        if ((rc = scd_launch_fp(g, p, q_user, q_il, batch, 0, g->n_angles, pack, L.pack_bytes, st, it > 0 ? &up : nullptr,
+                                w_il))) return rc;
         BpEpilogue e1;
         e1.c_acc = gs; e1.add1 = p; e1.c1 = 1.f; e1.add2 = nullptr; e1.c2 = 0.f;
         e1.out2 = nullptr; e1.dot_part = pd; e1.dot_stride = ps; e1.dot_with_add1 = 1;
@@ -146,7 +150,7 @@ int scd_cg_run(const scd_geom *g, const float *x_in, float *x, const float *rhs,
 // partial sums and beta live in the workspace.  With one sample per group (batch 1) an il image IS the reference
 // layout, so the caller's tensors are used directly and the update kernel is the reference-layout one.
 static int cg_run_il(const scd_geom *g, const CgLayout &L, const float *x_in, float *x, const float *b, float gamma,
-                     int n_iter, int batch, char *w, cudaStream_t st)
+                     int n_iter, int batch, char *w, cudaStream_t st, const float *w_il)
 {
     float *q = (float *)(w + L.il_q), *r = (float *)(w + L.il_r);
     float *p = (float *)(w + L.il_p), *d = (float *)(w + L.il_d);
@@ -164,7 +168,7 @@ static int cg_run_il(const scd_geom *g, const CgLayout &L, const float *x_in, fl
     const int na = g->n_angles;
     int rc;
     // r = b - x - gamma A*(A x);  rr = ||r||^2
-    if ((rc = scd_launch_fp_ilimg(g, x_in, nullptr, q, batch, 0, na, st, nullptr))) return rc;
+    if ((rc = scd_launch_fp_ilimg(g, x_in, nullptr, q, batch, 0, na, st, nullptr, w_il))) return rc;
     BpEpilogue e0;
     e0.il = 1; e0.mode = 0;
     e0.c_acc = -gs; e0.add1 = x_in; e0.c1 = -1.f; e0.add2 = b; e0.c2 = 1.f;
@@ -177,7 +181,7 @@ static int cg_run_il(const scd_geom *g, const CgLayout &L, const float *x_in, fl
         FpAccumulate acc;
         acc.rr_new_part = rr_new; acc.rr_new_n = rr_new_n; acc.rr_old_part = rr_old; acc.rr_old_n = rr_old_n;
         acc.part_stride = ps; acc.beta_out = beta;
-        if ((rc = scd_launch_fp_ilimg(g, r, nullptr, q, batch, 0, na, st, it > 0 ? &acc : nullptr))) return rc;
+        if ((rc = scd_launch_fp_ilimg(g, r, nullptr, q, batch, 0, na, st, it > 0 ? &acc : nullptr, w_il))) return rc;
         // p = r + beta p;  d = p + gamma A*(q);  pd = <p,d>
         BpEpilogue e1;
         e1.il = 1; e1.mode = 1;
@@ -211,9 +215,33 @@ static int cg_check(const scd_geom *g, const void *work, size_t work_bytes, int 
     return 0;
 }
 
+// packed measurement weights: 128-byte aligned like every sino_il buffer (the projector reads them as vectors)
+static int w_il_ok(const float *w_il, const char *who)
+{
+    if (((uintptr_t)w_il & 127) != 0) { scd_set_error("%s: w_il must be 128-byte aligned", who); return SCD_E_INVALID; }
+    return 0;
+}
+
+extern "C" int scd_sino_weights_pack(const scd_geom_t *g, const float *w, float *w_il, int batch, void *stream)
+{
+    if (!g || !w || !w_il) { scd_set_error("scd_sino_weights_pack: null argument"); return SCD_E_INVALID; }
+    if (batch <= 0) { scd_set_error("scd_sino_weights_pack: empty batch"); return SCD_E_INVALID; }
+    int rc = w_il_ok(w_il, "scd_sino_weights_pack");
+    if (rc) return rc;
+    // the view weights of A* are applied by the projector's output scale: the pack must not apply them again
+    return scd_launch_sino_pack(g, w, w_il, batch, 0, g->n_angles, (cudaStream_t)stream, false);
+}
+
 extern "C" int scd_cg(const scd_geom_t *g, float *x, const float *rhs, double gamma, int n_iter,
                       int batch, void *work, size_t work_bytes, void *stream)
 {
+    return scd_cg_w(g, x, rhs, nullptr, gamma, n_iter, batch, work, work_bytes, stream);
+}
+
+extern "C" int scd_cg_w(const scd_geom_t *g, float *x, const float *rhs, const float *w_il, double gamma, int n_iter,
+                        int batch, void *work, size_t work_bytes, void *stream)
+{
+    if (w_il && w_il_ok(w_il, "scd_cg_w")) return SCD_E_INVALID;
     if (g && x && rhs && work && batch > 0 && scd_il_image_ok(g, batch)) {
         const CgLayout L = cg_layout(g, batch);
         int rc = cg_check(g, work, work_bytes, n_iter, L, "scd_cg");
@@ -222,13 +250,13 @@ extern "C" int scd_cg(const scd_geom_t *g, float *x, const float *rhs, double ga
         char *w = (char *)work;
         cudaStream_t st = (cudaStream_t)stream;
         if (scd_group_samples(g, batch) == 1 && (((uintptr_t)x | (uintptr_t)rhs) & 15) == 0)
-            return cg_run_il(g, L, x, x, rhs, (float)gamma, n_iter, batch, w, st);      // the layouts coincide: in place
+            return cg_run_il(g, L, x, x, rhs, (float)gamma, n_iter, batch, w, st, w_il);      // the layouts coincide: in place
         float *xi = (float *)(w + L.il_x), *bi = (float *)(w + L.il_b);
         if ((rc = scd_launch_il_pack(g, x, xi, rhs, bi, batch, st))) return rc;
-        if ((rc = cg_run_il(g, L, xi, xi, bi, (float)gamma, n_iter, batch, w, st))) return rc;
+        if ((rc = cg_run_il(g, L, xi, xi, bi, (float)gamma, n_iter, batch, w, st, w_il))) return rc;
         return scd_launch_il_unpack(g, xi, x, batch, st);
     }
-    return scd_cg_run(g, x, x, rhs, (float)gamma, n_iter, batch, work, work_bytes, (cudaStream_t)stream, nullptr);
+    return scd_cg_run(g, x, x, rhs, (float)gamma, n_iter, batch, work, work_bytes, (cudaStream_t)stream, nullptr, w_il);
 }
 
 extern "C" size_t scd_fp_scratch_bytes(const scd_geom_t *g, int batch)
@@ -251,8 +279,16 @@ extern "C" size_t scd_sino_il_buffer_bytes(const scd_geom_t *g, int batch)
 extern "C" int scd_fp_il(const scd_geom_t *g, const float *img, float *sino_il, int batch,
                          int angle_lo, int angle_hi, void *scratch, size_t scratch_bytes, void *stream)
 {
+    return scd_fp_il_w(g, img, sino_il, nullptr, batch, angle_lo, angle_hi, scratch, scratch_bytes, stream);
+}
+
+extern "C" int scd_fp_il_w(const scd_geom_t *g, const float *img, float *sino_il, const float *w_il, int batch,
+                           int angle_lo, int angle_hi, void *scratch, size_t scratch_bytes, void *stream)
+{
     if (((uintptr_t)sino_il & 127) != 0) { scd_set_error("scd_fp_il: sino_il must be 128-byte aligned"); return SCD_E_INVALID; }
-    return scd_launch_fp(g, img, nullptr, sino_il, batch, angle_lo, angle_hi, scratch, scratch_bytes, (cudaStream_t)stream);
+    if (w_il && w_il_ok(w_il, "scd_fp_il_w")) return SCD_E_INVALID;
+    return scd_launch_fp(g, img, nullptr, sino_il, batch, angle_lo, angle_hi, scratch, scratch_bytes, (cudaStream_t)stream,
+                         nullptr, w_il);
 }
 
 extern "C" int scd_bp_il(const scd_geom_t *g, const float *sino_il, float *out, int batch,
@@ -307,10 +343,17 @@ extern "C" int scd_img_il_unpack(const scd_geom_t *g, const float *img_il, float
 extern "C" int scd_fp_ilimg(const scd_geom_t *g, const float *img_il, float *sino_il, int batch,
                             int angle_lo, int angle_hi, void *stream)
 {
+    return scd_fp_ilimg_w(g, img_il, sino_il, nullptr, batch, angle_lo, angle_hi, stream);
+}
+
+extern "C" int scd_fp_ilimg_w(const scd_geom_t *g, const float *img_il, float *sino_il, const float *w_il, int batch,
+                              int angle_lo, int angle_hi, void *stream)
+{
     int rc = il_args_ok(g, img_il, sino_il, batch, "scd_fp_ilimg");
     if (rc || batch == 0) return rc;
     if (((uintptr_t)sino_il & 127) != 0) { scd_set_error("scd_fp_ilimg: sino_il must be 128-byte aligned"); return SCD_E_INVALID; }
-    return scd_launch_fp_ilimg(g, img_il, nullptr, sino_il, batch, angle_lo, angle_hi, (cudaStream_t)stream, nullptr);
+    if (w_il && w_il_ok(w_il, "scd_fp_ilimg_w")) return SCD_E_INVALID;
+    return scd_launch_fp_ilimg(g, img_il, nullptr, sino_il, batch, angle_lo, angle_hi, (cudaStream_t)stream, nullptr, w_il);
 }
 
 extern "C" int scd_bp_ilimg(const scd_geom_t *g, const float *sino_il, float *out_il, int batch,
@@ -375,6 +418,17 @@ extern "C" int scd_dds_step(const scd_geom_t *g, const float *x, const float *s,
                             float *x_next, float *xhat0, int batch, void *work, size_t work_bytes,
                             void *stream)
 {
+    return scd_dds_step_w(g, x, s, atb, nullptr, eps, t, t_prev, abar, n_table, gamma, eta, n_iter, x_next, xhat0, batch,
+                          work, work_bytes, stream);
+}
+
+extern "C" int scd_dds_step_w(const scd_geom_t *g, const float *x, const float *s, const float *atb, const float *w_il,
+                              const float *eps, const float *t, const float *t_prev,
+                              const float *abar, int n_table, double gamma, double eta, int n_iter,
+                              float *x_next, float *xhat0, int batch, void *work, size_t work_bytes,
+                              void *stream)
+{
+    if (w_il && w_il_ok(w_il, "scd_dds_step_w")) return SCD_E_INVALID;
     if (!g || !x || !s || !atb || !eps || !t || !t_prev || !abar || !x_next || !xhat0 || !work) {
         scd_set_error("scd_dds_step: null argument"); return SCD_E_INVALID;
     }
@@ -396,12 +450,12 @@ extern "C" int scd_dds_step(const scd_geom_t *g, const float *x, const float *s,
             // one sample per group: il image = reference layout.  xhat0 (returned to the caller) is the start iterate,
             // read only; the first update writes the iterate into the workspace
             if ((rc = scd_launch_tweedie_rhs(x, s, atb, t, abar, n_table, (float)gamma, xhat0, bi, batch, (int64_t)L.img, st))) return rc;
-            if (n_iter > 0 && (rc = cg_run_il(g, L, xhat0, xi, bi, (float)gamma, n_iter, batch, w, st))) return rc;
+            if (n_iter > 0 && (rc = cg_run_il(g, L, xhat0, xi, bi, (float)gamma, n_iter, batch, w, st, w_il))) return rc;
             return scd_launch_ddim(n_iter > 0 ? xi : xhat0, s, eps, t, t_prev, abar, n_table, (float)eta, (float)(eta * eta),
                                    x_next, batch, (int64_t)L.img, st);
         }
         if ((rc = scd_launch_tweedie_il(g, x, s, atb, t, abar, n_table, (float)gamma, xhat0, xi, bi, batch, st))) return rc;
-        if (n_iter > 0 && (rc = cg_run_il(g, L, xi, xi, bi, (float)gamma, n_iter, batch, w, st))) return rc;
+        if (n_iter > 0 && (rc = cg_run_il(g, L, xi, xi, bi, (float)gamma, n_iter, batch, w, st, w_il))) return rc;
         return scd_launch_ddim_il(g, xi, s, eps, t, t_prev, abar, n_table, (float)eta, (float)(eta * eta), x_next, batch, st);
     }
     float *b = (float *)(w + L.off_b), *xh = (float *)(w + L.off_xh);
@@ -412,7 +466,7 @@ extern "C" int scd_dds_step(const scd_geom_t *g, const float *x, const float *s,
     memset(&tw, 0, sizeof(tw));
     tw.mode = 2; tw.x = x; tw.s = s; tw.atb = atb; tw.t = t; tw.abar = abar; tw.n_table = n_table;
     tw.gamma = (float)gamma; tw.xhat0 = xhat0; tw.b = b;
-    if ((rc = scd_cg_run(g, xhat0, xh, b, (float)gamma, n_iter, batch, work, work_bytes, st, &tw))) return rc;
+    if ((rc = scd_cg_run(g, xhat0, xh, b, (float)gamma, n_iter, batch, work, work_bytes, st, &tw, w_il))) return rc;
     return scd_launch_ddim(xh, s, eps, t, t_prev, abar, n_table, (float)eta, (float)(eta * eta), x_next,
                            batch, numel, st);
 }

@@ -73,6 +73,7 @@ struct MqParams {
     const float2  *rayt;     // [order position][n_det] (u0 + 1, b) per ray
     const float2  *angt;     // [order position] (scale, angle id bits)
     const float   *angw;     // [order position] view weight of the interleaved output (A* quadrature) or NULL
+    const float   *w_il;     // measurement weights W in the layout of sino_il (scd_sino_weights_pack) or NULL
     const int     *order;
     int n0, n1, n_angles, n_det, batch;
     int NA;                  // largest number of angles per CTA (sizes the tables)
@@ -673,7 +674,14 @@ fp_march_kernel(const MqParams P, const __grid_constant__ CUtensorMap tm0, const
             float *of = reinterpret_cast<float *>(&ov);
 #pragma unroll
             for (int v = 0; v < V; ++v) of[v] = sum[v] * sc;
-            VT *qp = reinterpret_cast<VT *>(dst + ((size_t)ang[ai].id * P.il_nb + P.il_padl + j) * SB + q * V);
+            const size_t qi = ((size_t)ang[ai].id * P.il_nb + P.il_padl + j) * SB + q * V;
+            VT *qp = reinterpret_cast<VT *>(dst + qi);
+            if (P.w_il) {                           // W A: per sample and bin, same place, same reason
+                const VT wv = __ldg(reinterpret_cast<const VT *>(P.w_il + (size_t)grp * ((size_t)P.n_angles * P.il_nb * SB) + qi));
+                const float *wf = reinterpret_cast<const float *>(&wv);
+#pragma unroll
+                for (int v = 0; v < V; ++v) of[v] *= wf[v];
+            }
             if (P.acc_mode) {                       // q = A r + beta * q_old
                 const VT old = *qp;
                 const float *pf = reinterpret_cast<const float *>(&old);
@@ -1113,7 +1121,7 @@ static void mq_fill_params(const scd_geom *g, const MqConfig &c, MqParams &P, fl
 // pack pass (producer fused in) + march over 1-D bulk copies
 int scd_launch_fp_v4(const scd_geom *g, const float *img, float *sino, float *sino_il, int batch,
                      int angle_lo, int angle_hi, void *scratch, size_t scratch_bytes, cudaStream_t st,
-                     const FpPrologue *prologue)
+                     const FpPrologue *prologue, const float *w_il)
 {
     FpPrologue Q;
     if (prologue) Q = *prologue; else { memset(&Q, 0, sizeof(Q)); }
@@ -1130,7 +1138,7 @@ int scd_launch_fp_v4(const scd_geom *g, const float *img, float *sino, float *si
     }
     MqParams P;
     mq_fill_params(g, c, P, sino, sino_il, batch, ncls);
-    P.img = img; P.packed = (float *)sp;
+    P.img = img; P.packed = (float *)sp; P.w_il = w_il;
 
     // ---- pack: image -> tile-ready layout (both orientations), producer fused in ----
     {
@@ -1154,7 +1162,7 @@ int scd_launch_fp_v4(const scd_geom *g, const float *img, float *sino, float *si
 // Tensor-copy path: project a sample-interleaved image img_il[group][k0][k1][SB] (SB = scd_group_samples >= 4) --
 // one launch, no packed copy.  acc != nullptr: q = A img + beta * q_old (see MqParams).
 int scd_launch_fp_ilimg(const scd_geom *g, const float *img_il, float *sino, float *sino_il, int batch,
-                        int angle_lo, int angle_hi, cudaStream_t st, const FpAccumulate *acc)
+                        int angle_lo, int angle_hi, cudaStream_t st, const FpAccumulate *acc, const float *w_il)
 {
     if (g && batch == 0) return 0;
     if (!g || !img_il || (!sino && !sino_il)) { scd_set_error("scd_fp: null argument"); return SCD_E_INVALID; }
@@ -1171,7 +1179,7 @@ int scd_launch_fp_ilimg(const scd_geom *g, const float *img_il, float *sino, flo
     if (c.smem > (size_t)g->smem_optin || !c.NSLOT) { scd_set_error("scd_fp: image too large for the shared-memory strip"); return SCD_E_INVALID; }
     MqParams P;
     mq_fill_params(g, c, P, sino, sino_il, batch, ncls);
-    P.img = img_il; P.zero_row = g->d_zero_row; P.lead = mq_lead(c.SB);
+    P.img = img_il; P.zero_row = g->d_zero_row; P.lead = mq_lead(c.SB); P.w_il = w_il;
     if (acc) {
         P.acc_mode = 1;
         P.rr_new_part = acc->rr_new_part; P.rr_new_n = acc->rr_new_n;
@@ -1218,7 +1226,7 @@ size_t scd_il_image_bytes(const scd_geom *g, int batch)
 // ------------------------------------------------------------- entry point ---
 int scd_launch_fp(const scd_geom *g, const float *img, float *sino, float *sino_il, int batch,
                   int angle_lo, int angle_hi, void *scratch, size_t scratch_bytes, cudaStream_t st,
-                  const FpPrologue *prologue)
+                  const FpPrologue *prologue, const float *w_il)
 {
     if (g && batch == 0) return 0;                 // empty batch: nothing to do (pointers may be null)
     if (!g || (!img && !(prologue && prologue->mode != 0)) || (!sino && !sino_il)) { scd_set_error("scd_fp: null argument"); return SCD_E_INVALID; }
@@ -1239,12 +1247,12 @@ int scd_launch_fp(const scd_geom *g, const float *img, float *sino, float *sino_
             return SCD_E_WORKSPACE;
         }
         if (SB == 1 && ((uintptr_t)img & 15) == 0)      // one sample per group: the image already is its interleaved form
-            return scd_launch_fp_ilimg(g, img, sino, sino_il, batch, angle_lo, angle_hi, st, nullptr);
+            return scd_launch_fp_ilimg(g, img, sino, sino_il, batch, angle_lo, angle_hi, st, nullptr, w_il);
         int rc = scd_launch_il_pack(g, img, (float *)sp, nullptr, nullptr, batch, st);
         if (rc) return rc;
-        return scd_launch_fp_ilimg(g, (const float *)sp, sino, sino_il, batch, angle_lo, angle_hi, st, nullptr);
+        return scd_launch_fp_ilimg(g, (const float *)sp, sino, sino_il, batch, angle_lo, angle_hi, st, nullptr, w_il);
     }
-    return scd_launch_fp_v4(g, img, sino, sino_il, batch, angle_lo, angle_hi, scratch, scratch_bytes, st, prologue);
+    return scd_launch_fp_v4(g, img, sino, sino_il, batch, angle_lo, angle_hi, scratch, scratch_bytes, st, prologue, w_il);
 }
 
 size_t scd_fp_scratch_need(const scd_geom *g, int batch)

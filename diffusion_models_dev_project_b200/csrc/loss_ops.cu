@@ -6,7 +6,8 @@
 //
 // i.e. both difference images are cropped to (H-1) x (W-1).  The reference evaluates this with
 // ~10 eager tensor passes forward and as many in autograd's backward; here
-//   residual_sq : r = Ax - y and the per-block partial sums of r^2 in one pass
+//   residual_sq : r = Ax - y and the per-block partial sums of r^2 in one pass; with measurement weights W
+//                 (PWLS, loss mean(W (Ax - y)^2)) r = W (Ax - y) and the partial sums of W (Ax - y)^2
 //   tv_fwd      : per-block partial sums of the cropped |dh| + |dw|
 //   tv_grad     : d tv / dx in one pass (sign(0) = 0 like torch.abs' backward)
 // Partial sums are written per block and added by the caller in index order (deterministic).
@@ -31,8 +32,8 @@ __device__ __forceinline__ float loss_block_sum(float v, float *red)
 }
 
 __global__ void __launch_bounds__(LOSS_THREADS)
-residual_sq_kernel(const float *__restrict__ ax, const float *__restrict__ y, float *__restrict__ r,
-                   float *__restrict__ part, int64_t numel)
+residual_sq_kernel(const float *__restrict__ ax, const float *__restrict__ y, const float *__restrict__ w,
+                   float *__restrict__ r, float *__restrict__ part, int64_t numel)
 {
     __shared__ float red[LOSS_THREADS / 32];
     scd_pdl_wait();
@@ -40,8 +41,9 @@ residual_sq_kernel(const float *__restrict__ ax, const float *__restrict__ y, fl
     float acc = 0.f;
     for (int64_t i = (int64_t)blockIdx.x * LOSS_THREADS + threadIdx.x; i < numel; i += (int64_t)gridDim.x * LOSS_THREADS) {
         const float d = ax[i] - y[i];
-        r[i] = d;
-        acc = fmaf(d, d, acc);
+        const float rw = w ? w[i] * d : d;         // W = 1: the same bits as no weights
+        r[i] = rw;
+        acc = fmaf(rw, d, acc);
     }
     const float tot = loss_block_sum(acc, red);
     if (threadIdx.x == 0) part[blockIdx.x] = tot;
@@ -96,14 +98,27 @@ static int loss_blocks(int64_t n)
 
 extern "C" int scd_residual_sq_blocks(int64_t numel) { return loss_blocks(numel); }
 
-extern "C" int scd_residual_sq(const float *ax, const float *y, float *r, float *part, int64_t numel, void *stream)
+int scd_launch_residual_sq(const float *ax, const float *y, const float *w, float *r, float *part, int64_t numel,
+                           cudaStream_t st)
 {
     if (!ax || !y || !r || !part) { scd_set_error("scd_residual_sq: null argument"); return SCD_E_INVALID; }
     if (numel <= 0) return 0;
-    SCD_CUDA(scd_launch_kernel(residual_sq_kernel, dim3(loss_blocks(numel)), dim3(LOSS_THREADS), 0, (cudaStream_t)stream, 0,
-                               ax, y, r, part, numel));
+    SCD_CUDA(scd_launch_kernel(residual_sq_kernel, dim3(loss_blocks(numel)), dim3(LOSS_THREADS), 0, st, 0,
+                               ax, y, w, r, part, numel));
     SCD_LAUNCH_CHECK("residual_sq_kernel");
     return 0;
+}
+
+extern "C" int scd_residual_sq(const float *ax, const float *y, float *r, float *part, int64_t numel, void *stream)
+{
+    return scd_launch_residual_sq(ax, y, nullptr, r, part, numel, (cudaStream_t)stream);
+}
+
+extern "C" int scd_residual_sq_w(const float *ax, const float *y, const float *w, float *r, float *part, int64_t numel,
+                                 void *stream)
+{
+    if (!w) { scd_set_error("scd_residual_sq_w: null weights"); return SCD_E_INVALID; }
+    return scd_launch_residual_sq(ax, y, w, r, part, numel, (cudaStream_t)stream);
 }
 
 extern "C" int scd_tv_blocks(int n0, int n1)

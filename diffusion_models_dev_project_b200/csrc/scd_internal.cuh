@@ -162,10 +162,11 @@ struct FpPrologue {
     float *xhat0, *b;
 };
 // sino: user layout [batch][n_angles][n_det] (may be NULL); sino_il: sample-interleaved layout read
-// by scd_launch_bp_il (may be NULL)
+// by scd_launch_bp_il (may be NULL); w_il: measurement weights in the layout of sino_il (scd_launch_sino_pack,
+// unweighted) that multiply the sino_il output only, or NULL
 int scd_launch_fp(const scd_geom *g, const float *img, float *sino, float *sino_il, int batch,
                   int angle_lo, int angle_hi, void *scratch, size_t scratch_bytes,
-                  cudaStream_t st, const FpPrologue *prologue = nullptr);
+                  cudaStream_t st, const FpPrologue *prologue = nullptr, const float *w_il = nullptr);
 // samples interleaved per pixel / detector bin for this batch (1, 2, 4, 8 or 16)
 int scd_group_samples(const scd_geom *g, int batch);
 
@@ -180,7 +181,8 @@ struct FpAccumulate {
     float *beta_out;
 };
 int scd_launch_fp_ilimg(const scd_geom *g, const float *img_il, float *sino, float *sino_il, int batch,
-                        int angle_lo, int angle_hi, cudaStream_t st, const FpAccumulate *acc);
+                        int angle_lo, int angle_hi, cudaStream_t st, const FpAccumulate *acc,
+                        const float *w_il = nullptr);
 // user layout -> il image for up to two arrays in one launch (b_user / b_il may be NULL)
 int scd_launch_il_pack(const scd_geom *g, const float *a_user, float *a_il, const float *b_user, float *b_il,
                        int batch, cudaStream_t st);
@@ -202,7 +204,7 @@ int scd_launch_cg_update_xr_il(const scd_geom *g, const float *x_in, float *x, f
 size_t scd_fp_scratch_need(const scd_geom *g, int batch);
 int scd_launch_fp_v4(const scd_geom *g, const float *img, float *sino, float *sino_il, int batch,
                      int angle_lo, int angle_hi, void *scratch, size_t scratch_bytes,
-                     cudaStream_t st, const FpPrologue *prologue);
+                     cudaStream_t st, const FpPrologue *prologue, const float *w_il = nullptr);
 size_t scd_fp_scratch_need_v4(const scd_geom *g, int batch);
 
 // Backprojection with fused epilogue:
@@ -270,7 +272,10 @@ int scd_launch_ddim(const float *xhat, const float *s, const float *eps,
                     int n_table, float eta, float eta2, float *out, int batch,
                     int64_t numel, cudaStream_t st);
 
-// x_in: start iterate (read only), x_out: result (may alias x_in)
+// x_in: start iterate (read only), x_out: result (may alias x_in); w_il: packed measurement weights or NULL
 int scd_cg_run(const scd_geom *g, const float *x_in, float *x_out, const float *rhs,
                float gamma, int n_iter, int batch, void *work, size_t work_bytes,
-               cudaStream_t st, const FpPrologue *first = nullptr);
+               cudaStream_t st, const FpPrologue *first = nullptr, const float *w_il = nullptr);
+// r = ax - y (w == NULL) or r = w (ax - y); part[k] = block-k partial sum of r (ax - y); all [numel] user layout
+int scd_launch_residual_sq(const float *ax, const float *y, const float *w, float *r, float *part, int64_t numel,
+                           cudaStream_t st);

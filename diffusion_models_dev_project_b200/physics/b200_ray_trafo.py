@@ -11,6 +11,7 @@ All arithmetic runs in hand-written sm_100a kernels reached through the C ABI
 must live on a CUDA device -- there is no CPU path.
 """
 import ctypes as C
+import math
 import threading
 from math import pi
 
@@ -102,21 +103,124 @@ class _AdjointFn(torch.autograd.Function):
         return (ag if w is None else ag * w), None
 
 
+class MeasurementWeights:
+    """Per-measurement weights ``W`` of the data-consistency system (penalised weighted least squares):
+    ``op(v) = v + gamma A*(W A v)``, ``rhs = xhat0 + gamma A*(W y)`` and the adaptation loss
+    ``mean(W (A x - y)^2) + lambda tv(x)``.  Low-dose data weighs each bin by its photon count (the inverse of the
+    variance of its log); a weight of 0 drops a measurement (dead bins, a metal trace, a view missing from one scan
+    of a batch).  The view weights of the geometry stay inside A*; ``W`` comes on top of them.
+
+    ``w``: float32 CUDA tensor of shape ``[..., n_angles, n_det]`` with at most two leading dimensions that broadcast
+    to those of the observations ``[B, C]``: ``[n_angles, n_det]`` or ``[1, 1, ...]`` (one map for every sample),
+    ``[B, 1, ...]`` (one per sample), ``[B, C, ...]``; finite and >= 0.  It is validated once here (one host read) and
+    copied, so that every path -- the fused calls, which read a packed copy, and the tensor expressions, which read
+    ``.w`` -- sees the same weights whatever later happens to the caller's tensor.  The packed copy in the projector's
+    sinogram layout is made once per observation shape (and launch tuning) and cached; the fused calls then take it
+    with no extra launch.  Build one object and pass it to every call: a plain tensor is validated and packed anew by
+    each call it is given to."""
+
+    def __init__(self, ray_trafo, w: Tensor):
+        if not isinstance(ray_trafo, B200RayTrafo):
+            raise TypeError('measurement weights need a B200RayTrafo (got %s); the angle-sharded operator does not '
+                            'take them' % type(ray_trafo).__name__)
+        if not isinstance(w, Tensor):
+            raise TypeError('measurement weights: a torch.Tensor is required (got %s)' % type(w).__name__)
+        if w.dtype != torch.float32:
+            raise TypeError('measurement weights: float32 required, got %s' % w.dtype)
+        obs = tuple(ray_trafo.obs_shape)
+        if not 2 <= w.dim() <= 4 or tuple(w.shape[-2:]) != obs:
+            raise ValueError('measurement weights: expected shape (*lead, *%r) with at most two leading dimensions, '
+                             'got %r' % (obs, tuple(w.shape)))
+        if not bool((torch.isfinite(w) & (w >= 0)).all()):
+            raise ValueError('measurement weights must be finite and >= 0')
+        if not w.is_cuda:
+            raise ValueError('measurement weights must live on a CUDA device (got %s)' % w.device)
+        self.ray_trafo = ray_trafo
+        self.w = w.detach().clone(memory_format=torch.contiguous_format)
+        self._cache = {}
+
+    def _lead(self, lead):
+        """The leading shape of the observations ``lead`` (checked: ``W`` broadcasts to it)."""
+        lead = tuple(int(d) for d in lead)
+        wl = tuple(self.w.shape[:-2])
+        if math.prod(wl) == 1:
+            return lead
+        try:
+            ok = torch.broadcast_shapes(wl, lead) == lead
+        except RuntimeError:
+            ok = False
+        if not ok:
+            raise ValueError('measurement weights of leading shape %r do not broadcast to observations of leading '
+                             'shape %r' % (wl, lead))
+        return lead
+
+    def expanded(self, lead) -> Tensor:
+        """``W`` as a contiguous ``[prod(lead), n_angles, n_det]`` tensor: the layout of observations whose leading
+        dimensions are ``lead`` (cached)."""
+        lead = self._lead(lead)
+        key = ('user', lead)
+        if key not in self._cache:
+            obs, batch = tuple(self.ray_trafo.obs_shape), math.prod(lead)
+            if math.prod(self.w.shape[:-2]) == 1:
+                w = self.w.reshape(1, *obs).expand(batch, *obs)
+            else:
+                w = self.w.expand(*lead, *obs).reshape(batch, *obs)
+            self._cache[key] = w.contiguous()
+        return self._cache[key]
+
+    def packed(self, lead, device) -> int:
+        """Device address of ``W`` packed for observations of leading shape ``lead`` (scd_sino_weights_pack; cached
+        per shape and launch tuning -- the layout depends on both; copies made under an earlier tuning are dropped)."""
+        if torch.device(device) != self.w.device:
+            raise ValueError('measurement weights live on %s, the operands on %s' % (self.w.device, device))
+        rt = self.ray_trafo
+        lead = self._lead(lead)
+        key = ('il', lead, rt._tuning_epoch)
+        hit = self._cache.get(key)
+        if hit is None:
+            for k in [k for k in self._cache if k[0] == 'il' and k[2] != rt._tuning_epoch]:
+                del self._cache[k]
+            w = self.expanded(lead)
+            batch = w.shape[0]
+            h = rt._handle(w.device)
+            buf = torch.empty(int(h._lib.scd_sino_il_buffer_bytes(h.ptr, batch)) + 256, dtype=torch.uint8, device=w.device)
+            ptr, _ = rt._aligned(buf)
+            with torch.cuda.device(w.device):
+                _lib.check(h._lib.scd_sino_weights_pack(h.ptr, w.data_ptr(), ptr, batch, _stream_ptr(w.device)),
+                           'scd_sino_weights_pack')
+            hit = self._cache[key] = (buf, ptr)
+        return hit[1]
+
+
+def as_weights(ray_trafo, weights):
+    """``None``, a :class:`MeasurementWeights` of ``ray_trafo``, or a tensor to wrap in one."""
+    if weights is None or isinstance(weights, MeasurementWeights):
+        if weights is not None and weights.ray_trafo is not ray_trafo:
+            raise ValueError('measurement weights were made for another ray transform')
+        return weights
+    return MeasurementWeights(ray_trafo, weights)
+
+
 class NormalOp:
     """``op(v) = v + gamma * A*(A v)`` -- the closure every predictor of the
     reference builds (reference src/samplers/utils.py:188-189, 235-236, 302-303),
     as an object so that :func:`..utils.cg.cg` can recognise it and run the
-    fused CUDA solve.  Calling it evaluates the operator (autograd-aware)."""
+    fused CUDA solve.  Calling it evaluates the operator (autograd-aware).
+    With ``weights`` (a :class:`MeasurementWeights` or a tensor for one) it is ``v + gamma * A*(W A v)``."""
 
-    def __init__(self, ray_trafo, gamma: float):
+    def __init__(self, ray_trafo, gamma: float, weights=None):
         self.ray_trafo = ray_trafo
         self.gamma = float(gamma)
+        self.weights = as_weights(ray_trafo, weights)
 
     def __call__(self, v: Tensor) -> Tensor:
         rt = self.ray_trafo
         if isinstance(rt, B200RayTrafo) and not (torch.is_grad_enabled() and v.requires_grad):
-            return rt.normal_apply(v, self.gamma)
-        return v + self.gamma * rt.trafo_adjoint(rt(v))
+            return rt.normal_apply(v, self.gamma, weights=self.weights)
+        av = rt(v)
+        if self.weights is not None:
+            av = self.weights.w * av
+        return v + self.gamma * rt.trafo_adjoint(av)
 
 
 class B200RayTrafo(BaseRayTrafo):
@@ -183,6 +287,7 @@ class B200RayTrafo(BaseRayTrafo):
         self._handles = {}
         self._work = {}
         self._weights = {}
+        self._tuning_epoch = 0          # bumped by set_tuning: packed measurement weights depend on the launch tuning
         self._hlock = threading.Lock()
 
     # ------------------------------------------------------------ plumbing ---
@@ -218,6 +323,7 @@ class B200RayTrafo(BaseRayTrafo):
     def set_tuning(self, device, **kw):
         """Override launch heuristics (see scd_set_tuning)."""
         h = self._handle(torch.device(device))
+        self._tuning_epoch += 1
         for k, v in kw.items():
             _lib.check(h._lib.scd_set_tuning(h.ptr, k.encode(), int(v)), 'scd_set_tuning')
 
@@ -326,9 +432,9 @@ class B200RayTrafo(BaseRayTrafo):
                                      _stream_ptr(y.device)), 'scd_bp')
         return x
 
-    def _fp_il(self, x: Tensor, angle_range=None) -> Tensor:
-        """A x in the library's sample-interleaved sinogram layout (opaque byte buffer, cached per
-        device and batch: valid until the next ``_fp_il`` of the same batch size)."""
+    def _fp_il(self, x: Tensor, angle_range=None, weights=None) -> Tensor:
+        """A x (``W A x`` with measurement weights) in the library's sample-interleaved sinogram layout (opaque byte
+        buffer, cached per device and batch: valid until the next ``_fp_il`` of the same batch size)."""
         x = self._prep(x, self.im_shape, 'trafo')
         h = self._handle(x.device)
         batch = int(np.prod(x.shape[:-2])) if x.dim() > 2 else 1
@@ -340,9 +446,10 @@ class B200RayTrafo(BaseRayTrafo):
             self._cache_put(key, buf)
         bp, _ = self._aligned(buf)
         scr = self.fp_scratch(batch, x.device)
+        wp = weights.packed(x.shape[:-2], x.device) if weights is not None else None
         with torch.cuda.device(x.device):
-            _lib.check(h._lib.scd_fp_il(h.ptr, x.data_ptr(), bp, batch, lo, hi, scr.data_ptr(), scr.numel(),
-                                        _stream_ptr(x.device)), 'scd_fp_il')
+            _lib.check(h._lib.scd_fp_il_w(h.ptr, x.data_ptr(), bp, wp, batch, lo, hi, scr.data_ptr(), scr.numel(),
+                                          _stream_ptr(x.device)), 'scd_fp_il_w')
         return buf
 
     def _bp_il(self, buf: Tensor, lead, scale: float, addend: Tensor = None, addend_scale: float = 0.0,
@@ -428,12 +535,13 @@ class B200RayTrafo(BaseRayTrafo):
         return out
 
     def normal_apply(self, v: Tensor, gamma: float, angle_range=None, add_identity: bool = True,
-                     out: Tensor = None) -> Tensor:
+                     out: Tensor = None, weights=None) -> Tensor:
         """``v + gamma*A*(A v)``: the projector writes the sinogram in the layout the backprojector
         stages from, the axpy is fused into the backprojector's epilogue (no grad).  ``out``: write the
-        result into this tensor (may not alias ``v``)."""
+        result into this tensor (may not alias ``v``).  ``weights`` (:class:`MeasurementWeights` or a tensor):
+        ``v + gamma*A*(W A v)``, W applied by the projector's output phase."""
         v = self._prep(v, self.im_shape, 'normal_apply')
-        q = self._fp_il(v, angle_range)
+        q = self._fp_il(v, angle_range, weights=as_weights(self, weights))
         return self._bp_il(q, v.shape[:-2], gamma * self.adj_scale, addend=v if add_identity else None,
                            addend_scale=1.0 if add_identity else 0.0, angle_range=angle_range, out=out)
 
@@ -498,13 +606,14 @@ class B200RayTrafo(BaseRayTrafo):
     trafo_flat = BaseRayTrafo._trafo_flat_via_trafo
     trafo_adjoint_flat = BaseRayTrafo._trafo_adjoint_flat_via_trafo_adjoint
 
-    def normal_op(self, gamma: float) -> NormalOp:
-        return NormalOp(self, gamma)
+    def normal_op(self, gamma: float, weights=None) -> NormalOp:
+        return NormalOp(self, gamma, weights)
 
     # ------------------------------------------------------------- solvers ---
-    def cg_solve(self, x0: Tensor, rhs: Tensor, gamma: float, n_iter: int) -> Tensor:
+    def cg_solve(self, x0: Tensor, rhs: Tensor, gamma: float, n_iter: int, weights=None) -> Tensor:
         """Fused batched CG on ``(I + gamma A*A) x = rhs`` from ``x0`` (no grad).
-        Same recurrences as the reference's ``cg`` (src/utils/cg.py:11-39)."""
+        Same recurrences as the reference's ``cg`` (src/utils/cg.py:11-39).  ``weights``: the system
+        ``(I + gamma A*WA)`` (:class:`MeasurementWeights`); ``rhs`` is the caller's, e.g. ``x0 + gamma A*(W y)``."""
         x0 = self._prep(x0, self.im_shape, 'cg x')
         rhs = self._prep(rhs, self.im_shape, 'cg rhs')
         if rhs.shape != x0.shape:
@@ -513,18 +622,21 @@ class B200RayTrafo(BaseRayTrafo):
             raise ValueError('cg: x and rhs live on different devices')
         h = self._handle(x0.device)
         batch = int(np.prod(x0.shape[:-2])) if x0.dim() > 2 else 1
+        weights = as_weights(self, weights)
+        wil = weights.packed(x0.shape[:-2], x0.device) if weights is not None else None
         x = x0.clone()
         w = self.workspace(batch, x0.device)
         wp, wn = self._aligned(w)
         with torch.cuda.device(x0.device):
-            _lib.check(h._lib.scd_cg(h.ptr, x.data_ptr(), rhs.data_ptr(), float(gamma), int(n_iter), batch,
-                                     wp, wn, _stream_ptr(x0.device)), 'scd_cg')
+            _lib.check(h._lib.scd_cg_w(h.ptr, x.data_ptr(), rhs.data_ptr(), wil, float(gamma), int(n_iter), batch,
+                                       wp, wn, _stream_ptr(x0.device)), 'scd_cg_w')
         return x
 
     def dds_step(self, x: Tensor, s: Tensor, atb: Tensor, eps: Tensor, t: Tensor, t_prev: Tensor,
-                 abar: Tensor, gamma: float, eta: float, n_iter: int):
+                 abar: Tensor, gamma: float, eta: float, n_iter: int, weights=None):
         """Tweedie -> rhs -> CG -> DDIM in one library call; returns ``(x_next, xhat0)``
-        (reference src/samplers/utils.py:195-218)."""
+        (reference src/samplers/utils.py:195-218).  ``weights``: CG on ``(I + gamma A*WA)``
+        (:class:`MeasurementWeights`); ``atb`` is then ``A*(W y)``."""
         x = self._prep(x, self.im_shape, 'dds x')
         s = self._prep(s, self.im_shape, 'dds s')
         atb = self._prep(atb, self.im_shape, 'dds rhs')
@@ -540,15 +652,17 @@ class B200RayTrafo(BaseRayTrafo):
         if t.numel() != batch or t_prev.numel() != batch:
             raise ValueError('dds_step: time steps must have one entry per sample')
         h = self._handle(x.device)
+        weights = as_weights(self, weights)
+        wil = weights.packed(x.shape[:-2], x.device) if weights is not None else None
         x_next = torch.empty_like(x)
         xhat0 = torch.empty_like(x)
         w = self.workspace(batch, x.device)
         wp, wn = self._aligned(w)
         with torch.cuda.device(x.device):
-            _lib.check(h._lib.scd_dds_step(
-                h.ptr, x.data_ptr(), s.data_ptr(), atb.data_ptr(), eps.data_ptr(), t.data_ptr(),
+            _lib.check(h._lib.scd_dds_step_w(
+                h.ptr, x.data_ptr(), s.data_ptr(), atb.data_ptr(), wil, eps.data_ptr(), t.data_ptr(),
                 t_prev.data_ptr(), abar.data_ptr(), int(abar.numel()), float(gamma), float(eta), int(n_iter),
-                x_next.data_ptr(), xhat0.data_ptr(), batch, wp, wn, _stream_ptr(x.device)), 'scd_dds_step')
+                x_next.data_ptr(), xhat0.data_ptr(), batch, wp, wn, _stream_ptr(x.device)), 'scd_dds_step_w')
         return x_next, xhat0
 
     # ----------------------------------------------------------------- fbp ---

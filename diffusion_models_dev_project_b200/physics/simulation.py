@@ -1,4 +1,5 @@
-"""Measurement simulation ``y = A x + white noise`` (reference src/physics/simulation.py:12-74)."""
+"""Measurement simulation ``y = A x + white noise`` (reference src/physics/simulation.py:12-74) and low-dose
+Poisson data with its statistical weights (:func:`simulate_poisson`)."""
 from typing import Any, Iterator, Optional, Tuple
 
 import numpy as np
@@ -24,6 +25,31 @@ def simulate(x: Tensor, ray_trafo, white_noise_rel_stddev: float, rng=None,
     noise = (z.to(observation.device) * noise_level).to(dtype=observation.dtype)
     noisy_observation = observation + noise
     return (noisy_observation, noise_level.item()) if return_noise_level else noisy_observation
+
+
+def simulate_poisson(x: Tensor, ray_trafo, photons: float, mu: float, rng: np.random.Generator,
+                     min_count: float = 0.1):
+    """Low-dose transmission data: photon counts ``N ~ Poisson(photons * exp(-mu * A x))`` per detector bin, the
+    log-transformed line integrals ``y = -log(max(N, min_count) / photons) / mu`` and their statistical weights.
+
+    ``mu`` scales the image to attenuation per unit length of the geometry; ``min_count`` replaces empty bins before
+    the log (a bin that saw no photon has no finite line integral).  After the log the variance of a bin is about
+    ``1 / (mu^2 N)``, so the penalised weighted least-squares weights are ``W = max(N, min_count)``, returned
+    normalised to mean 1 per sample so that ``gamma`` keeps its meaning.  The counts are drawn on the host from the
+    numpy generator ``rng`` (pass a seeded one for reproducible data): one read-back of ``A x``, outside any sampling
+    loop.  Returns ``(y, W)``, float32 of ``A x``'s shape on ``x``'s device; pass ``W`` as ``weights=`` to the
+    data-consistency calls (:class:`~.b200_ray_trafo.MeasurementWeights`)."""
+    if not (photons > 0 and mu > 0 and min_count > 0):
+        raise ValueError('simulate_poisson: photons, mu and min_count must be > 0')
+    ax = ray_trafo(x)
+    lam = float(photons) * np.exp(-float(mu) * ax.detach().to(torch.float64).cpu().numpy())
+    counts = np.maximum(rng.poisson(lam), float(min_count))
+    y = -np.log(counts / float(photons)) / float(mu)
+    per_sample = counts.reshape(counts.shape[0], -1).mean(axis=1).reshape(-1, *([1] * (counts.ndim - 1)))
+    w = counts / per_sample
+    dev = ax.device
+    return (torch.from_numpy(y).to(device=dev, dtype=torch.float32),
+            torch.from_numpy(w).to(device=dev, dtype=torch.float32))
 
 
 class SimulatedDataset(torch.utils.data.Dataset):

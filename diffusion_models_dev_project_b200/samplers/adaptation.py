@@ -16,10 +16,11 @@ class _AdaptationLossFn(torch.autograd.Function):
     """``mean((A x - y)^2) + lam * tv_loss(x)`` with hand-written forward and backward:
     A and the residual/TV reductions forward (5 launches), ``d tv/dx`` and one backprojection
     with the TV gradient as fused addend backward (3 launches).  The gradient through A follows the
-    ODL ``OperatorFunction`` pairing used everywhere else: ``(2/N) * A*(r) / c_w`` (SURVEY.md 8b)."""
+    ODL ``OperatorFunction`` pairing used everywhere else: ``(2/N) * A*(r) / c_w`` (SURVEY.md 8b).
+    With measurement weights ``wts`` the data term is ``mean(W (A x - y)^2)`` and ``r = W (A x - y)``."""
 
     @staticmethod
-    def forward(ctx, x, y, rt, lam):
+    def forward(ctx, x, y, rt, lam, wts=None):
         import ctypes as C
         from .. import _lib
         lib = _lib.load()
@@ -34,8 +35,13 @@ class _AdaptationLossFn(torch.autograd.Function):
         images = x.numel() // (rt.im_shape[0] * rt.im_shape[1])
         tvp = torch.empty(images * int(lib.scd_tv_blocks(*rt.im_shape)), dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
-            _lib.check(lib.scd_residual_sq(ax.data_ptr(), y.data_ptr(), r.data_ptr(), part.data_ptr(), numel, stream),
-                       'scd_residual_sq')
+            if wts is None:
+                _lib.check(lib.scd_residual_sq(ax.data_ptr(), y.data_ptr(), r.data_ptr(), part.data_ptr(), numel, stream),
+                           'scd_residual_sq')
+            else:
+                w = wts.expanded(x.shape[:-2])
+                _lib.check(lib.scd_residual_sq_w(ax.data_ptr(), y.data_ptr(), w.data_ptr(), r.data_ptr(), part.data_ptr(),
+                                                 numel, stream), 'scd_residual_sq_w')
             _lib.check(lib.scd_tv_loss(x.data_ptr(), tvp.data_ptr(), images, rt.im_shape[0], rt.im_shape[1], stream),
                        'scd_tv_loss')
         ctx.save_for_backward(x, r)
@@ -60,30 +66,38 @@ class _AdaptationLossFn(torch.autograd.Function):
         scale = 2.0 / ctx.numel * rt.adj_scale / rt.geometry.range_weight
         w = rt._view_weights(dev)
         grad = rt._bp(r if w is None else r / w, scale, addend=tvg, addend_scale=ctx.lam)
-        return grad * g, None, None, None
+        return grad * g, None, None, None, None
 
 
-def adaptation_loss(x, observation, ray_trafo, tv_penalty: float):
+def adaptation_loss(x, observation, ray_trafo, tv_penalty: float, weights=None):
     """The SCD adaptation loss (reference src/utils/exp_utils.py:256-257).  With a
     :class:`B200RayTrafo` and CUDA tensors it runs as fused kernels with a hand-written
-    backward; any other ray transform evaluates the reference's tensor expression."""
-    from ..physics.b200_ray_trafo import B200RayTrafo
+    backward; any other ray transform evaluates the reference's tensor expression.
+    ``weights`` (a :class:`MeasurementWeights` or a tensor): ``mean(W (A x - y)^2) + tv_penalty * tv(x)``."""
+    from ..physics.b200_ray_trafo import B200RayTrafo, MeasurementWeights, as_weights
     if isinstance(ray_trafo, B200RayTrafo) and x.is_cuda and x.dtype == torch.float32:
-        return _AdaptationLossFn.apply(x, observation, ray_trafo, float(tv_penalty))
-    return torch.mean((ray_trafo(x) - observation).pow(2)) + float(tv_penalty) * tv_loss(x)
+        return _AdaptationLossFn.apply(x, observation, ray_trafo, float(tv_penalty), as_weights(ray_trafo, weights))
+    res2 = (ray_trafo(x) - observation).pow(2)
+    if weights is not None:
+        res2 = (weights.w if isinstance(weights, MeasurementWeights) else weights) * res2
+    return torch.mean(res2) + float(tv_penalty) * tv_loss(x)
 
 
 class AdaptationLoss:
     """The loss closure of ``get_standard_adapted_sampler`` (reference src/utils/exp_utils.py:256-257) as an
     object, so that :func:`..samplers.utils._adapt` can recognise it and evaluate Tweedie -> data consistency ->
     loss and the whole backward sweep as two library calls (``scd_adapt_fwd`` / ``scd_adapt_bwd``).  Calling it
-    evaluates the loss at ``x`` like the reference's lambda."""
+    evaluates the loss at ``x`` like the reference's lambda.  ``weights``: measurement weights ``W`` of the data
+    term, ``mean(W (A x - y)^2)`` (:class:`MeasurementWeights` or a tensor for one); the data-consistency step of
+    the adaptation objective then solves ``(I + gamma A*WA)`` as well."""
 
-    def __init__(self, observation, ray_trafo, tv_penalty: float):
+    def __init__(self, observation, ray_trafo, tv_penalty: float, weights=None):
+        from ..physics.b200_ray_trafo import B200RayTrafo, as_weights
         self.observation, self.ray_trafo, self.tv_penalty = observation, ray_trafo, float(tv_penalty)
+        self.weights = as_weights(ray_trafo, weights) if isinstance(ray_trafo, B200RayTrafo) else weights
 
     def __call__(self, x):
-        return adaptation_loss(x, self.observation, self.ray_trafo, self.tv_penalty)
+        return adaptation_loss(x, self.observation, self.ray_trafo, self.tv_penalty, self.weights)
 
 
 _DC_CODES = {'cg': 0, 'dc': 1, 'gd': 1, 'none': 2}
@@ -95,7 +109,7 @@ class _AdaptObjectiveFn(torch.autograd.Function):
     CG recurrences exactly, as autograd does for the reference (src/samplers/utils.py:241-260)."""
 
     @staticmethod
-    def forward(ctx, s, x, t, atb, y, rt, abar, gamma, n_iter, dc_code, lam):
+    def forward(ctx, s, x, t, atb, y, rt, abar, gamma, n_iter, dc_code, lam, wts):
         import ctypes as C
         from .. import _lib
         lib = _lib.load()
@@ -116,12 +130,14 @@ class _AdaptObjectiveFn(torch.autograd.Function):
         wp = work.data_ptr() + (-work.data_ptr()) % 256
         loss = torch.empty((), dtype=torch.float32, device=dev)
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        w_user = wts.expanded(x.shape[:-2]).data_ptr() if wts is not None else None
+        w_il = wts.packed(x.shape[:-2], dev) if wts is not None else None
         with torch.cuda.device(dev):
-            _lib.check(lib.scd_adapt_fwd(h.ptr, x.data_ptr(), s.data_ptr(), atb.data_ptr() if atb is not None else None,
-                                         y.data_ptr(), t.data_ptr(), abar.data_ptr(), int(abar.numel()), float(gamma),
-                                         int(n_iter), int(dc_code), float(lam), loss.data_ptr(), None, batch, wp, n_work,
-                                         stream), 'scd_adapt_fwd')
-        ctx.rt, ctx.work, ctx.wp, ctx.n_work, ctx.batch = rt, work, wp, n_work, batch
+            _lib.check(lib.scd_adapt_fwd_w(h.ptr, x.data_ptr(), s.data_ptr(), atb.data_ptr() if atb is not None else None,
+                                           y.data_ptr(), w_user, w_il, t.data_ptr(), abar.data_ptr(), int(abar.numel()),
+                                           float(gamma), int(n_iter), int(dc_code), float(lam), loss.data_ptr(), None, batch,
+                                           wp, n_work, stream), 'scd_adapt_fwd_w')
+        ctx.rt, ctx.work, ctx.wp, ctx.n_work, ctx.batch, ctx.w_il = rt, work, wp, n_work, batch, w_il
         ctx.t, ctx.abar = t, abar
         ctx.args = (float(gamma), int(n_iter), int(dc_code), float(lam))
         ctx.shape = s.shape
@@ -143,12 +159,13 @@ class _AdaptObjectiveFn(torch.autograd.Function):
         g = g.to(device=dev, dtype=torch.float32).contiguous()
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         with torch.cuda.device(dev):
-            _lib.check(lib.scd_adapt_bwd(h.ptr, g.data_ptr(), ctx.t.data_ptr(), ctx.abar.data_ptr(), int(ctx.abar.numel()),
-                                         # dx^2/ds: the mean cell cancels; the call backprojects without view weights
-                                         gamma, n_iter, dc_code, lam, rt.adj_scale / rt.geometry.range_weight,
-                                         grad_s.data_ptr(), ctx.batch, ctx.wp, ctx.n_work, stream), 'scd_adapt_bwd')
+            _lib.check(lib.scd_adapt_bwd_w(h.ptr, g.data_ptr(), ctx.w_il, ctx.t.data_ptr(), ctx.abar.data_ptr(),
+                                           int(ctx.abar.numel()),
+                                           # dx^2/ds: the mean cell cancels; the call backprojects without view weights
+                                           gamma, n_iter, dc_code, lam, rt.adj_scale / rt.geometry.range_weight,
+                                           grad_s.data_ptr(), ctx.batch, ctx.wp, ctx.n_work, stream), 'scd_adapt_bwd_w')
         ctx.work = None
-        return (grad_s,) + (None,) * 10
+        return (grad_s,) + (None,) * 11
 
 
 def adapt_objective_applies(x, rhs, loss_fn, sde, dc_type: str) -> bool:
@@ -172,7 +189,7 @@ def adapt_objective(s, x, time_step, rhs, loss_fn: 'AdaptationLoss', sde, gamma:
         return None
     return _AdaptObjectiveFn.apply(s, x, time_step, rhs, loss_fn.observation, loss_fn.ray_trafo,
                                    sde.alpha_bar_table(x.device), float(gamma), int(n_iter), _DC_CODES[dc_type],
-                                   loss_fn.tv_penalty)
+                                   loss_fn.tv_penalty, loss_fn.weights)
 
 
 def _score_model_adpt(score: nn.Module, impl: str = 'full', adpt_kwargs: Optional[Dict] = None,

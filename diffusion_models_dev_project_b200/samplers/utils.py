@@ -21,7 +21,7 @@ from torch import Tensor
 
 from .. import fused
 from .adaptation import adapt_objective, adapt_objective_applies
-from ..physics.b200_ray_trafo import B200RayTrafo, NormalOp
+from ..physics.b200_ray_trafo import B200RayTrafo, NormalOp, MeasurementWeights, as_weights
 from ..utils.cg import cg
 from ..utils.sde import SDE, VESDE, VPSDE, DDPM, _SCORE_PRED_CLASSES
 
@@ -45,10 +45,30 @@ def _fusable(sde, *tensors) -> bool:
     return True
 
 
-def _make_op(ray_trafo, gamma):
+def _make_op(ray_trafo, gamma, weights=None):
+    """``v + gamma A*(A v)``, or ``v + gamma A*(W A v)`` with measurement weights."""
     if isinstance(ray_trafo, B200RayTrafo):
-        return NormalOp(ray_trafo, gamma)
+        return NormalOp(ray_trafo, gamma, weights)
+    if weights is not None:
+        return lambda v: v + gamma * ray_trafo.trafo_adjoint(weights * ray_trafo(v))
     return lambda v: v + gamma * ray_trafo.trafo_adjoint(ray_trafo(v))
+
+
+def _dc_weights(ray_trafo, cg_kwargs):
+    """The measurement weights of the data consistency, ``cg_kwargs['weights']`` (None without).  Pass a
+    :class:`MeasurementWeights` (the factories do): a plain tensor is validated and packed on every call."""
+    weights = (cg_kwargs or {}).get('weights')
+    if weights is not None and isinstance(ray_trafo, B200RayTrafo):
+        weights = as_weights(ray_trafo, weights)
+    return weights
+
+
+def _weighted_gd(ray_trafo, xhat0, gamma, rhs, weights):
+    """One gradient step on the data term: ``xhat0 - gamma A*(W A xhat0) + gamma rhs`` (W = 1 without weights)."""
+    ax = ray_trafo(xhat0)
+    if weights is not None:
+        ax = (weights.w if isinstance(weights, MeasurementWeights) else weights) * ax
+    return xhat0 - gamma * ray_trafo.trafo_adjoint(ax) + gamma * rhs
 
 
 def apTweedy(s: Tensor, x: Tensor, sde: SDE, time_step: Tensor) -> Tensor:
@@ -103,7 +123,11 @@ def decomposed_diffusion_sampling_sde_predictor(
         use_simplified_eqn: bool = False, ray_trafo=None) -> Tuple[Tensor, Tensor]:
     """Decomposed diffusion sampling step: score -> Tweedie -> CG data consistency
     on ``(I + gamma A*A) x = xhat0 + gamma A*y`` -> DDIM.  Returns ``(x_next, xhat0)``
-    -- the second value is the Tweedie estimate, not the CG result (reference :218)."""
+    -- the second value is the Tweedie estimate, not the CG result (reference :218).
+    ``cg_kwargs['weights']`` (optional measurement weights W, :class:`MeasurementWeights` or a tensor): CG on
+    ``(I + gamma A*WA)``; ``rhs`` is then ``A*(W y)``.  (They ride in the solver options so that the predictor keeps
+    the reference's signature.)"""
+    weights = _dc_weights(ray_trafo, cg_kwargs)
     pair = isinstance(time_step, tuple)
     t = time_step[0] if pair else time_step
     with torch.no_grad():
@@ -112,9 +136,9 @@ def decomposed_diffusion_sampling_sde_predictor(
             eps = torch.randn_like(x)
             x_next, xhat0 = ray_trafo.dds_step(
                 x, s, rhs, eps, t, time_step[1], sde.alpha_bar_table(x.device),
-                gamma=gamma, eta=eta, n_iter=cg_kwargs['max_iter'])
+                gamma=gamma, eta=eta, n_iter=cg_kwargs['max_iter'], weights=weights)
             return x_next.detach(), xhat0.detach()
-        op = _make_op(ray_trafo, gamma)
+        op = _make_op(ray_trafo, gamma, weights)
         xhat0 = apTweedy(s=s, x=x, sde=sde, time_step=t)
         xhat = cg(op=op, x=xhat0, rhs=xhat0 + gamma * rhs, n_iter=cg_kwargs['max_iter'])
         x = ddim(sde=sde, s=s, xhat=xhat, time_step=time_step, step_size=step_size, eta=eta,
@@ -185,9 +209,12 @@ class _AdaptGraph:
         # the captured graph holds the observation by address: a loss object that is re-used with another
         # observation (or an address recycled after garbage collection) must not hit a stale graph
         obs = loss_fn.observation
+        # likewise the measurement weights (their packed copies are addressed by the graph)
+        wts = getattr(loss_fn, 'weights', None)
+        wkey = None if wts is None else (id(wts), wts.w.data_ptr(), wts.w._version)
         return (id(loss_fn), obs.data_ptr(), obs._version, tuple(obs.shape), loss_fn.tv_penalty, id(loss_fn.ray_trafo),
                 tuple(x.shape), x.device, None if rhs is None else tuple(rhs.shape), float(lr), float(gamma), int(n_iter),
-                dc_type)
+                dc_type, wkey)
 
     def reset(self):
         with torch.no_grad():
@@ -213,8 +240,12 @@ def _adapt(x: Tensor, score, sde: SDE, ray_trafo, loss_fn, time_step: Tensor, rh
 
     ``cuda_graph`` (default: environment variable ``SCD_ADAPT_CUDA_GRAPH=1``): capture one Adam step -- score
     model included -- in a CUDA graph and replay it (:class:`_AdaptGraph`); needs the fused objective (standard
-    adaptation loss on the CUDA operator) and a score model that is safe to capture."""
-    op = _make_op(ray_trafo, gamma)
+    adaptation loss on the CUDA operator) and a score model that is safe to capture.
+
+    Measurement weights ride on ``loss_fn`` (``AdaptationLoss(..., weights=W)``): the data-consistency step of the
+    objective then solves ``(I + gamma A*WA)`` and ``rhs`` is ``A*(W y)``."""
+    weights = getattr(loss_fn, 'weights', None)
+    op = _make_op(ray_trafo, gamma, weights)
     assert _has_lora_active(score=score)
     score.eval()
     if cuda_graph is None:
@@ -244,7 +275,7 @@ def _adapt(x: Tensor, score, sde: SDE, ray_trafo, loss_fn, time_step: Tensor, rh
         if dc_type == "cg":
             xhat = cg(op=op, x=xhat0, rhs=xhat0 + gamma * rhs, n_iter=n_iter)
         elif dc_type == "dc":
-            xhat = xhat0 - gamma * ray_trafo.trafo_adjoint(ray_trafo(xhat0)) + gamma * rhs
+            xhat = _weighted_gd(ray_trafo, xhat0, gamma, rhs, weights)
         elif dc_type == "none":
             xhat = xhat0
         else:
@@ -262,12 +293,15 @@ def adapted_ddim_sde_predictor(
         cg_kwargs: Dict = None, rhs: Tensor = None) -> Tuple[Tensor, Tensor]:
     """SCD step (reference :280-336): optional adaptation, Tweedie with the adapted
     score, optional data consistency (``cg`` | ``gd`` | ``none``), DDIM with the
-    un-adapted score (LoRA scale switched to 0 for that call)."""
+    un-adapted score (LoRA scale switched to 0 for that call).  ``cg_kwargs['weights']``: measurement weights W of
+    the data consistency, ``(I + gamma A*WA)`` (``rhs`` is then ``A*(W y)``); the adaptation takes them from its
+    loss."""
+    weights = _dc_weights(ray_trafo, cg_kwargs)
     pair = isinstance(time_step, tuple)
     t = time_step[0] if pair else time_step
     if use_adapt:
         adapt_fn(x=x, time_step=t, ray_trafo=ray_trafo, rhs=rhs, gamma=gamma, n_iter=cg_kwargs['max_iter'])
-    op = _make_op(ray_trafo, gamma)
+    op = _make_op(ray_trafo, gamma, weights)
     with torch.no_grad():
         s = score(x, t)
         xhat0 = apTweedy(s=s, x=x, sde=sde, time_step=t)
@@ -275,7 +309,7 @@ def adapted_ddim_sde_predictor(
             if dc_type == "cg":
                 xhat = cg(op=op, x=xhat0, rhs=xhat0 + gamma * rhs, n_iter=cg_kwargs['max_iter'])
             elif dc_type == "gd":
-                xhat = xhat0 - gamma * ray_trafo.trafo_adjoint(ray_trafo(xhat0)) + gamma * rhs
+                xhat = _weighted_gd(ray_trafo, xhat0, gamma, rhs, weights)
             elif dc_type == "none":
                 xhat = xhat0
             else:

@@ -208,7 +208,14 @@ class AngleShardedRayTrafo:
         self._reduce_chunks(produce, yf.shape[0], out)
         return out.reshape(*lead, *self.im_shape)
 
-    def normal_apply(self, v: Tensor, gamma: float) -> Tensor:
+    @staticmethod
+    def _no_weights(weights) -> None:
+        if weights is not None:
+            raise ValueError('AngleShardedRayTrafo does not take measurement weights: run the weighted '
+                             'data-consistency system on an unsharded B200RayTrafo')
+
+    def normal_apply(self, v: Tensor, gamma: float, weights=None) -> Tensor:
+        self._no_weights(weights)
         self._no_grad_only(v, 'normal_apply')
         lead = v.shape[:-2]
         vf = v.reshape(-1, 1, *self.im_shape)
@@ -233,7 +240,8 @@ class AngleShardedRayTrafo:
         self._reduce_chunks(produce, vf.shape[0], out)
         return out.reshape(*lead, *self.im_shape)
 
-    def normal_op(self, gamma: float):
+    def normal_op(self, gamma: float, weights=None):
+        self._no_weights(weights)
         return lambda v: self.normal_apply(v, gamma)
 
     def _peer_state(self, n_slices: int, device):

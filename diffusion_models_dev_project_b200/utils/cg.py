@@ -8,7 +8,8 @@ and, as in the reference, unused) and no guard against a zero residual.
 When ``op`` is a :class:`~..physics.b200_ray_trafo.NormalOp` on a
 :class:`B200RayTrafo` and no gradient is required, the whole solve runs as the
 fused CUDA launch sequence ``scd_cg`` (A, A* with the axpy and <p,d> in its
-epilogue, one update kernel, one direction kernel per iteration).  Any other
+epilogue, one update kernel, one direction kernel per iteration); a ``NormalOp``
+with measurement weights, ``v + gamma A*(W A v)``, takes the same path (``scd_cg_w``).  Any other
 callable -- and every call that must be differentiated, e.g. the LoRA
 adaptation of SCD (reference src/samplers/utils.py:241-260) -- runs the same
 recurrences as tensor operations on whatever device the tensors live on.
@@ -40,7 +41,8 @@ class _CgSelfAdjointFn(torch.autograd.Function):
 
     That holds for ``op(v) = v + gamma*A*(A v)`` on :class:`B200RayTrafo`: with ODL's gradient pairing
     (grad of ``trafo`` = ``A*(g)/c_w``, grad of ``trafo_adjoint`` = ``c_w*A(g)``, SURVEY.md 8b) the
-    gradient through ``op`` is ``g + gamma*A*(A g)``.  The forward pass runs the same recurrences as the
+    gradient through ``op`` is ``g + gamma*A*(A g)`` -- and ``g + gamma*A*(W A g)`` with measurement weights,
+    a diagonal between the two.  The forward pass runs the same recurrences as the
     tensor path below (same values), keeps ``p_k, d_k, r_{k+1}`` and the scalars of every iteration, and
     the backward pass differentiates them exactly -- the iterates are a non-linear function of ``x`` and
     ``rhs`` (alpha, beta), so this is NOT the adjoint linear solve -- with ``n_iter + 1`` operator
@@ -109,14 +111,14 @@ def _self_adjoint_nograd(op):
     """``op`` evaluated without recording a graph, when its gradient is known to be ``op`` itself."""
     from ..physics.b200_ray_trafo import B200RayTrafo, NormalOp
     if isinstance(op, NormalOp) and isinstance(op.ray_trafo, B200RayTrafo):
-        rt, gamma = op.ray_trafo, op.gamma
-        return lambda v: rt.normal_apply(v, gamma)
+        rt, gamma, weights = op.ray_trafo, op.gamma, op.weights
+        return lambda v: rt.normal_apply(v, gamma, weights=weights)
     return None
 
 
 def cg(op: callable, x: Tensor, rhs: Tensor, n_iter: int = 5, tol: float = 1e-10) -> Tensor:
     if _fused_ok(op, x, rhs):
-        return op.ray_trafo.cg_solve(x, rhs, op.gamma, n_iter)
+        return op.ray_trafo.cg_solve(x, rhs, op.gamma, n_iter, weights=op.weights)
     if torch.is_grad_enabled() and (x.requires_grad or rhs.requires_grad) and x.is_cuda and x.dim() == 4:
         op_nograd = _self_adjoint_nograd(op)
         if op_nograd is not None:

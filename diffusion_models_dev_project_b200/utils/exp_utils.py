@@ -16,7 +16,8 @@ from math import ceil
 import torch
 
 from .sde import VESDE, VPSDE, DDPM, _EPSILON_PRED_CLASSES
-from ..physics import B200RayTrafo, simulate
+from ..physics import B200RayTrafo, MeasurementWeights, simulate, simulate_poisson
+from ..physics.b200_ray_trafo import as_weights
 from ..physics.geometry import ParallelBeamGeometry2D
 from ..samplers import (BaseSampler, decomposed_diffusion_sampling_sde_predictor,
                         adapted_ddim_sde_predictor, tv_loss, adaptation_loss, AdaptationLoss, _adapt, _score_model_adpt,
@@ -79,18 +80,59 @@ def get_data_from_ground_truth(ground_truth, ray_trafo, white_noise_rel_stddev):
     return ground_truth, observation, filtbackproj
 
 
+def get_low_dose_data_from_ground_truth(ground_truth, ray_trafo, photons: float, mu: float, rng=None,
+                                        min_count: float = 0.1):
+    """Low-dose counterpart of :func:`get_data_from_ground_truth`: Poisson counts at ``photons`` incident photons per
+    bin (:func:`~..physics.simulation.simulate_poisson`).  Returns ``(ground_truth, observation, fbp, weights)``; pass
+    ``weights`` to :func:`get_standard_sampler` / :func:`get_standard_adapted_sampler`."""
+    import numpy as np
+    ground_truth = ground_truth.unsqueeze(0) if ground_truth.ndim == 3 else ground_truth
+    observation, weights = simulate_poisson(ground_truth, ray_trafo, photons, mu,
+                                            rng if rng is not None else np.random.default_rng(), min_count=min_count)
+    return ground_truth, observation, ray_trafo.fbp(observation), weights
+
+
+def _dc_weights(ray_trafo, weights):
+    """The weights the predictors get: on the CUDA operator one :class:`MeasurementWeights`, validated and packed
+    once for the whole run (a plain tensor would be validated and packed again on every step); else as given."""
+    return as_weights(ray_trafo, weights) if isinstance(ray_trafo, B200RayTrafo) else weights
+
+
+def _weighted_rhs(ray_trafo, observation, weights):
+    """``A*(y)``, or ``A*(W y)`` with measurement weights (the right-hand side of the weighted system)."""
+    if weights is None:
+        return ray_trafo.trafo_adjoint(observation)
+    return ray_trafo.trafo_adjoint((weights.w if isinstance(weights, MeasurementWeights) else weights) * observation)
+
+
+def _cg_kwargs(args, weights):
+    """The predictors' solver options; measurement weights ride there (the predictors keep the reference's
+    signatures)."""
+    kw = {'max_iter': int(args.cg_iter)}
+    if weights is not None:
+        kw['weights'] = weights
+    return kw
+
+
 def _im_shape_of(ray_trafo):
     return ray_trafo.im_shape if not hasattr(ray_trafo, 'resize') else ray_trafo.resize.shape
 
 
-def get_standard_sampler(args, config, score, sde, ray_trafo, observation=None, filtbackproj=None, device=None):
+def get_standard_sampler(args, config, score, sde, ray_trafo, observation=None, filtbackproj=None, device=None,
+                         weights=None):
     """Sampler factory with the reference's signature (src/utils/exp_utils.py:123-223).
 
     ``dds`` (the data-consistency hot path) for every schedule; ``dps`` = diffusion posterior
     sampling (Euler-Maruyama for VE/VP, ancestral for DDPM); ``naive`` = score + data-fit gradient
     (VE/VP only, as in the reference).  The reference passes an undefined ``init_chain_fn`` on the
-    VE/VP branch; here the chain always starts from the prior."""
+    VE/VP branch; here the chain always starts from the prior.
+
+    ``weights``: measurement weights ``W`` (e.g. of :func:`get_low_dose_data_from_ground_truth`), ``dds`` only: the
+    data consistency solves ``(I + gamma A*WA) x = xhat0 + gamma A*(W y)``."""
     method = args.method.lower()
+    if weights is not None and method != 'dds':
+        raise ValueError('measurement weights apply to the dds data-consistency step only (method %r)' % method)
+    weights = _dc_weights(ray_trafo, weights)
     shape = _im_shape_of(ray_trafo)
     eps_pred = any(isinstance(sde, c) for c in _EPSILON_PRED_CLASSES)
     sample_kwargs = {
@@ -109,7 +151,7 @@ def get_standard_sampler(args, config, score, sde, ray_trafo, observation=None, 
                                       'use_simplified_eqn': True, 'ray_trafo': ray_trafo}
         predictor = functools.partial(
             decomposed_diffusion_sampling_sde_predictor, score=score, sde=sde,
-            rhs=ray_trafo.trafo_adjoint(observation), cg_kwargs={'max_iter': int(args.cg_iter)})
+            rhs=_weighted_rhs(ray_trafo, observation, weights), cg_kwargs=_cg_kwargs(args, weights))
     elif method == 'dps' and eps_pred:
         sample_kwargs['predictor'] = {'penalty': float(args.penalty)}
         sample_kwargs['early_stopping_pct'] = float(args.early_stopping_pct)
@@ -128,7 +170,9 @@ def get_standard_sampler(args, config, score, sde, ray_trafo, observation=None, 
 
 
 def get_standard_adapted_sampler(args, config, score, sde, ray_trafo, observation=None, device=None,
-                                 complex_y=False, lora_inject_fn=None):
+                                 complex_y=False, lora_inject_fn=None, weights=None):
+    """``weights``: measurement weights ``W`` of the adaptation loss ``mean(W (A x - y)^2) + tv`` and of the data
+    consistency ``(I + gamma A*WA) x = xhat0 + gamma A*(W y)``."""
     if args.method.lower() != 'dds':
         raise NotImplementedError
     eps = getattr(config.sampling, 'eps', 0.)
@@ -150,15 +194,15 @@ def get_standard_adapted_sampler(args, config, score, sde, ray_trafo, observatio
         adpt_kwargs = {'include_blocks': args.lora_include_blocks, 'r': int(args.lora_rank)}
     _score_model_adpt(score, impl=args.adaptation, adpt_kwargs=adpt_kwargs, inject_fn=lora_inject_fn)
 
-    loss_fn = AdaptationLoss(observation, ray_trafo, float(args.tv_penalty))     # callable: loss_fn(x=...)
+    loss_fn = AdaptationLoss(observation, ray_trafo, float(args.tv_penalty), weights=weights)   # callable: loss_fn(x=...)
 
     adapt_fn = functools.partial(_adapt, score=score, sde=sde, loss_fn=loss_fn,
                                  num_steps=int(args.num_optim_step), lr=float(args.lr),
                                  cuda_graph=getattr(args, 'adapt_cuda_graph', None))
     predictor = functools.partial(
         adapted_ddim_sde_predictor, score=score, sde=sde, adapt_fn=adapt_fn, add_cg=args.add_cg,
-        dc_type=args.dc_type, rhs=ray_trafo.trafo_adjoint(observation),
-        cg_kwargs={'max_iter': int(args.cg_iter)})
+        dc_type=args.dc_type, rhs=_weighted_rhs(ray_trafo, observation, loss_fn.weights),
+        cg_kwargs=_cg_kwargs(args, loss_fn.weights))
     if any(isinstance(sde, c) for c in _EPSILON_PRED_CLASSES):
         try:
             tl, tr = config.sampling.travel_length, config.sampling.travel_repeat

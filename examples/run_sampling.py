@@ -12,6 +12,7 @@ data-consistency path, not a trained prior), a small LoRA injector instead of th
     python examples/run_sampling.py --num_steps 20 --angle_range 0 90        # limited angle: a 90 degree wedge
     python examples/run_sampling.py --num_steps 20 --angles_file views.txt   # sparse / non-uniform views
     python examples/run_sampling.py --num_steps 20 --adjoint matched         # A* = exact transpose of A
+    python examples/run_sampling.py --num_steps 20 --photons 1e4             # low-dose Poisson data, PWLS weights
 """
 import argparse
 import os
@@ -65,6 +66,11 @@ def parse():
     p.add_argument('--adjoint', default='pixel', choices=['pixel', 'matched'],
                    help="backprojector: 'pixel' (pixel-driven, SimpleTrafo's) or 'matched' (exact transpose of the "
                         "Joseph projector, MatmulRayTrafo's)")
+    p.add_argument('--photons', type=float, default=None,
+                   help='low dose: Poisson counts with this many incident photons per bin instead of white noise, '
+                        'reconstructed with the statistical weights W ~ counts (dds only)')
+    p.add_argument('--mu', type=float, default=0.01,
+                   help='--photons: attenuation per image unit and pixel length (A x of the phantoms reaches ~200)')
     p.add_argument('--batch_size', type=int, default=1)
     p.add_argument('--num_images', type=int, default=1)
     p.add_argument('--unet', default='small', choices=['small', 'aapm', 'blur'],
@@ -110,17 +116,24 @@ def main():
         ground_truth = phantoms[i:i + 1].to(device).expand(args.batch_size, -1, -1, -1).contiguous()
         torch.manual_seed(config.seed + i)
         np.random.seed(config.seed + i)
-        _, observation, filtbackproj = pkg.get_data_from_ground_truth(
-            ground_truth=ground_truth, ray_trafo=ray_trafo, white_noise_rel_stddev=config.data.stddev)
+        weights = None
+        if args.photons is not None:
+            _, observation, filtbackproj, weights = pkg.get_low_dose_data_from_ground_truth(
+                ground_truth=ground_truth, ray_trafo=ray_trafo, photons=args.photons, mu=args.mu,
+                rng=np.random.default_rng(config.seed + i))
+        else:
+            _, observation, filtbackproj = pkg.get_data_from_ground_truth(
+                ground_truth=ground_truth, ray_trafo=ray_trafo, white_noise_rel_stddev=config.data.stddev)
         if args.mode == 'conditional':
             sampler = pkg.get_standard_sampler(args=args, config=config, score=score, sde=sde, ray_trafo=ray_trafo,
-                                               observation=observation, filtbackproj=filtbackproj, device=device)
+                                               observation=observation, filtbackproj=filtbackproj, device=device,
+                                               weights=weights)
         else:
             args.method = 'dds'
             import copy
             sampler = pkg.get_standard_adapted_sampler(args=args, config=config, score=copy.deepcopy(score), sde=sde,
                                                        ray_trafo=ray_trafo, observation=observation, device=device,
-                                                       lora_inject_fn=inject_trainable_lora)
+                                                       lora_inject_fn=inject_trainable_lora, weights=weights)
         recon = sampler.sample(logging=False)
         psnr = pkg.PSNR(recon[0, 0].cpu().numpy(), ground_truth[0, 0].cpu().numpy())
         psnr_fbp = pkg.PSNR(filtbackproj[0, 0].cpu().numpy(), ground_truth[0, 0].cpu().numpy())

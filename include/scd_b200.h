@@ -151,6 +151,28 @@ int scd_fp_ilimg(const scd_geom_t *g, const float *img_il, float *sino_il, int b
 int scd_bp_ilimg(const scd_geom_t *g, const float *sino_il, float *out_il, int batch,
                  int angle_lo, int angle_hi, float c_acc, const float *addend_il, float c_add, void *stream);
 
+/* Measurement weights (penalised weighted least squares): a float32 weight per sample, view and bin,
+ *   W [batch][n_angles][n_det]   (user layout; finite and >= 0; 0 drops the measurement)
+ * turns the data-consistency system into  op(v) = v + gamma A*(W A v),  rhs = xhat0 + gamma A*(W y)  and the
+ * adaptation loss into  mean(W (A x - y)^2) + lambda tv(x).  The view weights of a weighted geometry stay inside A*;
+ * W comes on top of them.  scd_fp, scd_bp and scd_ramp_filter are never weighted.
+ *   scd_sino_weights_pack  W -> w_il, the sample-interleaved sinogram layout (scd_sino_il_buffer_bytes(g, batch)
+ *                          bytes, 128-byte aligned; zero pads).  Pack once per (W, batch size), outside the sampling
+ *                          loop; every _w call below takes w_il and multiplies the projector's interleaved output by
+ *                          it, before any recurrence (one more 16-byte load per output vector, no extra launch).
+ * Contracts (the library cannot check device data without a synchronisation):
+ *   - the caller guarantees that W is finite and >= 0;
+ *   - a w_il buffer is valid only for the batch size, and the "fp_samples" tuning (scd_set_tuning), it was packed
+ *     with, and only for the geometry that packed it.
+ * w_il == NULL in a _w call is the unweighted call; W == 1 gives the same bits as NULL (a multiply by 1.0f is exact).
+ * Calls with weights stay allocation-free, sync-free and graph-capturable.                                     */
+int scd_sino_weights_pack(const scd_geom_t *g, const float *w, float *w_il, int batch, void *stream);
+/* sino_il = W A img (scd_fp_il / scd_fp_ilimg with weights): A*(sino_il) is then A*(W A img), normal_apply's term */
+int scd_fp_il_w(const scd_geom_t *g, const float *img, float *sino_il, const float *w_il, int batch,
+                int angle_lo, int angle_hi, void *scratch, size_t scratch_bytes, void *stream);
+int scd_fp_ilimg_w(const scd_geom_t *g, const float *img_il, float *sino_il, const float *w_il, int batch,
+                   int angle_lo, int angle_hi, void *stream);
+
 /* Bytes of scratch scd_cg / scd_dds_step need for `batch` samples.           */
 size_t scd_cg_workspace_bytes(const scd_geom_t *g, int batch);
 
@@ -160,6 +182,10 @@ size_t scd_cg_workspace_bytes(const scd_geom_t *g, int batch);
  * (src/utils/cg.py:11-39, src/samplers/utils.py:188-189).                    */
 int scd_cg(const scd_geom_t *g, float *x, const float *rhs, double gamma,
            int n_iter, int batch, void *work, size_t work_bytes, void *stream);
+/* scd_cg on (I + gamma A*WA) x = rhs (w_il: scd_sino_weights_pack; NULL = scd_cg).  rhs = x0 + gamma A*(W y) is
+ * the caller's.                                                                                              */
+int scd_cg_w(const scd_geom_t *g, float *x, const float *rhs, const float *w_il, double gamma,
+             int n_iter, int batch, void *work, size_t work_bytes, void *stream);
 
 /* DDPM alpha-bar table: abar[k] = prod_{m<k}(1 - beta_m) rounded to fp32, k in
  * [0, n_table) with abar[0] = 1 (index t+1, so t = -1 -> 1).  Device pointer,
@@ -195,6 +221,11 @@ int scd_dds_step(const scd_geom_t *g, const float *x, const float *s,
                  double gamma, double eta, int n_iter, float *x_next,
                  float *xhat0, int batch, void *work, size_t work_bytes,
                  void *stream);
+/* scd_dds_step with CG on (I + gamma A*WA) (w_il: scd_sino_weights_pack; NULL = scd_dds_step); atb = A*(W y).  */
+int scd_dds_step_w(const scd_geom_t *g, const float *x, const float *s, const float *atb, const float *w_il,
+                   const float *eps, const float *t, const float *t_prev, const float *abar, int n_table,
+                   double gamma, double eta, int n_iter, float *x_next, float *xhat0, int batch, void *work,
+                   size_t work_bytes, void *stream);
 
 /* Adaptation loss of SCD, loss(x) = mean((A x - y)^2) + lambda*tv_loss(x)
  * (src/utils/exp_utils.py:256-257, src/samplers/adaptation.py:7-11):
@@ -204,6 +235,9 @@ int scd_dds_step(const scd_geom_t *g, const float *x, const float *s,
  * The caller adds the partials (in index order: deterministic).                */
 int scd_residual_sq_blocks(int64_t numel);
 int scd_residual_sq(const float *ax, const float *y, float *r, float *part, int64_t numel, void *stream);
+/* weighted residual: r = w (ax - y), part[k] = block-k partial sum of w (ax - y)^2 (w: [numel], finite, >= 0) */
+int scd_residual_sq_w(const float *ax, const float *y, const float *w, float *r, float *part, int64_t numel,
+                      void *stream);
 int scd_tv_blocks(int n0, int n1);
 int scd_tv_loss(const float *x, float *part, int images, int n0, int n1, void *stream);
 int scd_tv_grad(const float *x, float *grad, int images, int n0, int n1, void *stream);
@@ -228,6 +262,17 @@ int scd_adapt_fwd(const scd_geom_t *g, const float *x, const float *s, const flo
 int scd_adapt_bwd(const scd_geom_t *g, const float *grad_loss, const float *t, const float *abar, int n_table,
                   double gamma, int n_iter, int dc_type, double tv_lambda, double trafo_grad_scale,
                   float *grad_s, int batch, void *work, size_t work_bytes, void *stream);
+/* The objective with measurement weights: every application of op is v + gamma A*(W A v) (w_il) and the loss is
+ * mean(W (A xhat - y)^2) + tv_lambda tv(xhat) (w: [batch][n_angles][n_det], user layout).  atb = A*(W y).  The
+ * forward call keeps W (A xhat - y) in `work`, so the backward call needs only w_il; pass the same w_il to both.
+ * w and w_il are both NULL (the unweighted calls) or both given.                                             */
+int scd_adapt_fwd_w(const scd_geom_t *g, const float *x, const float *s, const float *atb, const float *y,
+                    const float *w, const float *w_il, const float *t, const float *abar, int n_table, double gamma,
+                    int n_iter, int dc_type, double tv_lambda, float *loss, float *xhat_out, int batch, void *work,
+                    size_t work_bytes, void *stream);
+int scd_adapt_bwd_w(const scd_geom_t *g, const float *grad_loss, const float *w_il, const float *t, const float *abar,
+                    int n_table, double gamma, int n_iter, int dc_type, double tv_lambda, double trafo_grad_scale,
+                    float *grad_s, int batch, void *work, size_t work_bytes, void *stream);
 
 /* Ramp filter of the filtered back-projection: every sinogram row is convolved along the detector
  * axis with the band-limited ramp (Kak & Slaney / the "ramp" Fourier filter of the reference's recipe)
